@@ -91,7 +91,13 @@ def parse():
     ap.add_argument("--no-graph", action="store_true", help="learner step launched eagerly instead of as one CUDA graph")
     ap.add_argument("--separate-streams", action="store_true", help="draw the index / goal streams in their own launch (fdql_sample_streams)")
     ap.add_argument("--tail-scan", action="store_true", help="relabelled returns by scanning the episode tail instead of the link records")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the batch, loss and d loss / d q_pred of the last timed pass as DIR/<name>.npy "
+                         "(a fixed, seeded sample of its windows); inputs are seeded, so two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA path computed: it needs --impl ours")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -458,6 +464,8 @@ def run_ours(args):
     parity = None
     if not args.no_parity_check and rank == 0:
         parity = oracle_spot_check(torch, ring, chk, z, q, lp, loss, grad, n, exact)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, args.dump_outputs, chk, loss, grad, n)
     loss_mean_timed, relabel_frac_timed = float(loss.mean()), float(chk["flags"].float().mean())
     if dist:
         dist.barrier()
@@ -979,6 +987,24 @@ def oracle_spot_check(torch, ring, b, z, q, lp, loss, grad, n, exact, n_check=10
                             "loss": rel(gl, ol[:, 0]), "grad_q_over_its_scale": float(np.max(np.abs(gg - og)) / max(np.abs(og).max(), 1e-30))},
             "tolerance": "bit-exact for indices, goals, done masks, steps; 1e-5 relative for returns, targets and losses",
             "ok": bool(sum(mism.values()) == 0 and rel(got["mc_return"], want["mc_return"]) < 1e-5 and rel(gl, ol[:, 0]) < 1e-5)}
+
+
+def dump_outputs(torch, d, b, loss, grad, n, n_sample=16384, seed=0):
+    """What the caller of the timed path receives for its last pass, as d/<name>.npy: the drawn streams (start row, hindsight
+    flag, goal row), the relabelled batch [T, windows, width] with its learner aux (mask, is_contiguous, loss_weight), and the
+    per-transition loss and d loss / d q_pred [T - 1, windows(, CQ)].  The whole pass is ~360 MB, so the same fixed, seeded
+    sample of `n_sample` windows (window_index) is taken from every array: ~23 MB.  Row indices are stored as float64 (exact)."""
+    os.makedirs(d, exist_ok=True)
+    idx = np.sort(np.random.default_rng(seed).choice(n, min(n_sample, n), replace=False))
+    it = torch.as_tensor(idx, device=loss.device)
+    arrays = {"window_index": torch.as_tensor(idx), "starts": b["starts"][it], "hindsight_flags": b["flags"][it],
+              "goal_rows": b["goals"][it]}
+    arrays.update((k, v[:, it]) for k, v in b["out"].items())
+    arrays.update(mask=b["mask"][:, it], is_contiguous=b["contig"][:, it], loss_weight=b["weight"][:, it],
+                  loss=loss.view(T - 1, n)[:, it], grad_q=grad.view(T - 1, n, CQ)[:, it])
+    for name, a in arrays.items():
+        a = a.cpu().numpy()
+        np.save(os.path.join(d, name + ".npy"), a.astype(np.float64 if a.dtype == np.int64 else np.float32))
 
 
 # ---------------------------------------------------------------------------------------------------------------------
