@@ -4,7 +4,7 @@ state equals the goal; reward -1 until then): vectorised numpy bit-flip envs -> 
 commit, link records) -> `Learner.train_step` (sample-time "future" hindsight relabelling, fused TQC loss, discrete Gumbel-softmax
 actor with the one-hot kernel, whole step as a CUDA graph).  Prints the greedy success rate as it trains.
 
-    python examples/train_bitflip_her.py --bits 10 --updates 4000
+    python examples/train_bitflip_her.py --bits 10 --updates 4000 [--per]
 """
 import argparse
 import os
@@ -60,6 +60,7 @@ def main():
     ap.add_argument("--envs", type=int, default=64)
     ap.add_argument("--batch", type=int, default=1024)
     ap.add_argument("--eps", type=float, default=0.2)
+    ap.add_argument("--per", action="store_true", help="prioritized replay (use_prioritized_replay=True)")
     args = ap.parse_args()
     device = torch.device("cuda:0")
     rng = np.random.default_rng(0)
@@ -68,7 +69,8 @@ def main():
     conf = Agent.LearnerConf(training_device="cuda:0", obs_space={"obs_1d": bits, "achieved_goal": bits, "desired_goal": bits},
                              action_space=types.SimpleNamespace(n=bits, shape=()), discrete=True, num_critics=5, num_q_predictions=10,
                              top_quantiles_to_drop=0.2, batch_size=args.batch, temporal_len=2, replay_size=200_000, use_HER=True,
-                             her_mode="future", num_instances=1, gamma=0.98, learning_rate=1e-3, use_cuda_graph=True)
+                             her_mode="future", num_instances=1, gamma=0.98, learning_rate=1e-3, use_cuda_graph=True,
+                             use_prioritized_replay=args.per, per_beta_steps=args.updates)
     read, write = Replay.make(conf, compute_reward=fdql.RewardOp.bitflip())
     learner = Agent.Learner(conf, read)
     actor = learner.actor_critic.actor

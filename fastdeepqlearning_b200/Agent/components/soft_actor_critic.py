@@ -52,17 +52,18 @@ class _LossWithStats(torch.autograd.Function):
 
 
 class _ReducedLossWithStats(torch.autograd.Function):
-    """sum_m weight[m] * loss[m] as one scalar; the kernel applied `weight` to d loss / d q_pred itself (grad_scale)."""
+    """sum_m weight[m] * loss[m] as one scalar; the kernel applied `weight` to d loss / d q_pred itself (grad_scale).  The unweighted
+    per-transition loss comes out as a third, non-differentiable output (the priority signal of prioritized replay)."""
 
     @staticmethod
     def forward(ctx, q_pred, fn, weight):
         r = fn(q_pred)
         ctx.save_for_backward(r["grad"])
-        ctx.mark_non_differentiable(r["stats"])
-        return (r["loss"] * weight).sum(), r["stats"]
+        ctx.mark_non_differentiable(r["stats"], r["loss"])
+        return (r["loss"] * weight).sum(), r["stats"], r["loss"]
 
     @staticmethod
-    def backward(ctx, g_total, _g_stats):
+    def backward(ctx, g_total, _g_stats, _g_loss):
         (grad,) = ctx.saved_tensors
         return grad * g_total, None, None
 
@@ -145,15 +146,17 @@ class SoftActorCritic(nn.Module):
         return ops.sac_min_target_loss(q_pred, next_z, lp, next_xp["reward"], next_xp["mask"], lb, self.curr_alpha, self.conf.gamma,
                                        grad_scale=grad_scale, want_stats=True)
 
-    def q_loss_reduced(self, curr_xp, next_xp, weight):
+    def q_loss_reduced(self, curr_xp, next_xp, weight, with_loss=False):
         """(sum over the [T-1, B] transitions of weight * q_loss, summaries): q_loss followed by the learner's loss reduce
-        (deepQlearning.py:222-225,249) with the reduce weights folded into the kernel's backward pass."""
+        (deepQlearning.py:222-225,249) with the reduce weights folded into the kernel's backward pass.  `with_loss=True` appends the
+        unweighted per-transition loss [T-1, B, 1] (detached) to the pair."""
         conf = self.conf
         q_pred, next_z, next_log_pi = self._critic_io(curr_xp, next_xp)
         lb = next_xp["mc_return"] if conf.use_nStep_lowerbounds else None
         lp = next_log_pi if conf.use_max_entropy_q else None
-        total, stats = _ReducedLossWithStats.apply(q_pred, lambda q: self._q_loss_fused(q, next_z, lp, next_xp, lb, weight), weight)
-        return total, _summaries_from_stats(stats, q_pred.shape[-1], lb is not None)
+        total, stats, loss = _ReducedLossWithStats.apply(q_pred, lambda q: self._q_loss_fused(q, next_z, lp, next_xp, lb, weight), weight)
+        summ = _summaries_from_stats(stats, q_pred.shape[-1], lb is not None)
+        return (total, summ, loss) if with_loss else (total, summ)
 
     def _alias_frozen_critic(self):
         """soft_actor_critic.py:142 copies critic -> critic_frozen before every actor update so that the policy gradient flows through

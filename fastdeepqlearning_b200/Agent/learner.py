@@ -23,7 +23,10 @@ class LearnerConf(types.SimpleNamespace):
                  num_q_predictions=10, top_quantiles_to_drop=0.2, use_max_entropy_q=True, use_distributional_sac=True,
                  use_squashed_rewards=False, num_instances=1, training_device="cuda:0", dtype=torch.float32,
                  init_log_alpha=0.0, learning_rate=3e-4, pi_hidden_dims=(256,), critic_hidden_dims=(256, 256), discrete=False,
-                 obs_keys=("obs_1d", "achieved_goal", "desired_goal"), use_bootstrap_minibatch_nstep=False, clip_grad_norm=None)
+                 obs_keys=("obs_1d", "achieved_goal", "desired_goal"), use_bootstrap_minibatch_nstep=False, clip_grad_norm=None,
+                 # prioritized replay (Schaul et al. 2016; not a reference mode): priority exponent, importance-sampling exponent annealed
+                 # linearly from per_beta0 to 1 over per_beta_steps updates, priority floor, max / mean mix over a window (R2D2)
+                 use_prioritized_replay=False, per_alpha=0.6, per_beta0=0.4, per_beta_steps=100_000, per_eps=1e-6, per_eta=0.9)
         d.update(kw)
         super().__init__(**d)
 
@@ -60,6 +63,8 @@ class Learner:
         self._buckets = None  # (critic parameters, all the others): the two gradient buckets of the split backward
         self._prefetched = {}  # replay -> batch sampled during the previous step's gradient all-reduce
         self.last_summaries = {}
+        self._per = bool(getattr(conf, "use_prioritized_replay", False))
+        self._priority_signal = None  # (starts, per-transition critic loss, is_contiguous) of the batch get_losses last saw
 
     def close(self):
         """Drop the captured step graphs.  Call before torch.distributed.destroy_process_group(): a CUDA graph that captured the
@@ -83,8 +88,12 @@ class Learner:
         """deepQlearning.py:198-249.  `xp` is a sampled [T, B, .] dict; it is mutated like in the reference (mask,
         is_contiguous, state).  When the gather kernel already emitted mask / is_contiguous (aux=True) they are used as is.
         `parts=True` (folded reduce only) returns (critic part, actor + temperature part) of the same scalar: their backward passes
-        touch disjoint parameters, which `_one_update` uses to overlap the critic gradients' all-reduce with the actor's backward."""
+        touch disjoint parameters, which `_one_update` uses to overlap the critic gradients' all-reduce with the actor's backward.
+        A prioritized batch (`is_weight` [B] and `starts` [B] in xp) weights the CRITIC loss of window b by is_weight[b], in the folded
+        path (grad_scale of the loss kernel) and the unfolded one alike; the actor and temperature losses keep the uniform reduce
+        weights.  The critic's per-transition loss is kept for update_priorities."""
         conf = self.conf
+        is_w, starts = xp.pop("is_weight", None), xp.pop("starts", None)
         if "mask" not in xp:
             xp["mask"] = torch.logical_not(xp["task_done"] != 0).to(xp["task_done"].dtype)
         if "is_contiguous" not in xp:
@@ -101,16 +110,25 @@ class Learner:
         if weight is not None and not bootstrap and getattr(conf, "fold_loss_reduce", True):
             # :222-225,249 folded into the loss kernel: the gather kernel's aux weight contig / ((sum_t contig + 1e-4) B T) goes in as
             # grad_scale, so d loss / d q_pred leaves the kernel already reduced and the scalar is sum(weight * per-transition loss)
-            q_sum, summ = self.actor_critic.q_loss_reduced(curr, nxt, weight)
+            if is_w is None:
+                q_sum, summ = self.actor_critic.q_loss_reduced(curr, nxt, weight)
+            else:
+                q_sum, summ, q_each = self.actor_critic.q_loss_reduced(curr, nxt, weight * is_w.view(1, -1, 1), with_loss=True)
+                self._priority_signal = (starts, q_each, is_contiguous)
             pi_loss, alpha_loss, asumm = self.actor_critic.actor_loss(curr)
             self.last_summaries = {**summ, **asumm, "Valid_Portion": is_contiguous.mean()}
             if parts:
                 return q_sum, ((pi_loss + alpha_loss) * weight).sum()
             return q_sum + ((pi_loss + alpha_loss) * weight).sum()
         if parts:
+            if is_w is not None:
+                xp["is_weight"], xp["starts"] = is_w, starts  # for the unsplit call that follows
             return None
         q_loss, bound, summ = self.actor_critic.q_loss(curr, nxt)
         pi_loss, alpha_loss, asumm = self.actor_critic.actor_loss(curr)
+        if is_w is not None:
+            self._priority_signal = (starts, q_loss.detach(), is_contiguous)
+            q_loss = q_loss * is_w.view(1, -1, 1)
         loss = ((q_loss + pi_loss + alpha_loss) * is_contiguous).sum(0) / (is_contiguous.sum(0) + 1e-4)   # :222-225
         loss = loss.mean()
         if bootstrap:                                                                                   # :226-228
@@ -142,6 +160,8 @@ class Learner:
         side stream while the main stream already samples and relabels the NEXT step's batch (SURVEY.md section 5: the only
         collective of the path hides behind work that does not depend on it); the prefetched batch is consumed by the next call."""
         key = id(replay)
+        if self._per:
+            sample_kw.setdefault("prioritized", True)
         xp = self._prefetched.pop(key, None)
         if xp is None:
             xp = replay.temporal_sample(**sample_kw)
@@ -150,6 +170,8 @@ class Learner:
         sb = getattr(self.conf, "split_backward", True)  # True: with the overlapped all-reduce; "force": always (tests); False: never
         if ((overlap and sb) or sb == "force") and self.device.type == "cuda" and not any(p.requires_grad for p in self.encoder.parameters()):
             split = self.get_losses(xp, parts=True)  # None when the reduce is not folded (then: one backward, one bucket)
+            if split is not None:
+                self._feed_priorities(replay)
         if split is not None:
             # critic gradients first; their all-reduce (most of the bytes) runs on the side stream under the actor's backward
             q_part, pi_part = split
@@ -178,6 +200,7 @@ class Learner:
             self.actor_critic.update_target()
             return loss
         loss = self.get_losses(xp)
+        self._feed_priorities(replay)
         loss.backward()
         if overlap:
             cur = torch.cuda.current_stream(self.device)
@@ -197,6 +220,28 @@ class Learner:
         self.actor_critic.update_target()
         return loss.detach()
 
+    def _feed_priorities(self, replay):
+        """update_priorities from the critic loss of the batch just consumed, enqueued before the next batch (or the prefetch) is drawn."""
+        if self._priority_signal is None:
+            return
+        starts, q_each, contig = self._priority_signal
+        self._priority_signal = None
+        replay.update_priorities(starts, q_each, contig)
+
+    def per_beta(self):
+        """Importance-sampling exponent of the current update: per_beta0 annealed linearly to 1 over per_beta_steps updates."""
+        c = self.conf
+        frac = min(1.0, self.train_steps / max(1, int(c.per_beta_steps)))
+        return float(c.per_beta0) + (1.0 - float(c.per_beta0)) * frac
+
+    @staticmethod
+    def _ring_of(replay):
+        """The ReplayMemory under a read head's wrappers."""
+        ring = replay
+        while hasattr(ring, "replay_buffer") or (hasattr(ring, "replay") and not hasattr(ring, "flush")):
+            ring = getattr(ring, "replay_buffer", None) or ring.replay
+        return getattr(ring, "replay", ring)
+
     @staticmethod
     def _world_size():
         import torch.distributed as dist
@@ -206,6 +251,8 @@ class Learner:
         """deepQlearning.py:105-127: for each local shard: sample -> loss -> backward -> (all-reduce) -> Adam -> targets."""
         last = None
         for i, replay in enumerate(self.replays):
+            if self._per:
+                self._ring_of(replay).set_priority_beta(self.per_beta())  # device scalar: read by the sampler, eager or replayed
             if getattr(self.conf, "use_cuda_graph", False):
                 last = self._graphed_update(i, replay)
             else:
@@ -217,10 +264,7 @@ class Learner:
     # ---- whole-step CUDA graph (SURVEY.md section 8f rank 2): sample/relabel kernel, MLP forward/backward, fused loss, Adam and
     #      the target update are captured once and replayed; the draw counter and the temperature live in device memory.
     def _graphed_update(self, i, replay):
-        ring = replay
-        while hasattr(ring, "replay_buffer") or (hasattr(ring, "replay") and not hasattr(ring, "flush")):
-            ring = getattr(ring, "replay_buffer", None) or ring.replay
-        ring = getattr(ring, "replay", ring)
+        ring = self._ring_of(replay)
         ring.flush()
         n_now = len(ring)
         entry = self._graphs.get(i)
@@ -232,6 +276,7 @@ class Learner:
                 raise RuntimeError("clip_grad_norm is not capturable")
             ring.device_counter = True  # draw counter AND ring length are read from device memory: one capture serves a filling ring
             ring.publish_len()
+            ring.apply_pending_priorities()  # rows recorded since the last PER call: applied outside the graph, never captured
             cur = torch.cuda.current_stream(self.device)
             side = torch.cuda.Stream(self.device)
             side.wait_stream(cur)
@@ -248,5 +293,6 @@ class Learner:
             entry = (graph, static_loss, n_now)
             self._graphs[i] = entry
         ring.publish_len()  # (a no-op unless rows were added since the last step)
+        ring.apply_pending_priorities()
         entry[0].replay()
         return entry[1]

@@ -13,6 +13,11 @@ def make(conf, **kwargs):
               for _ in range(conf.num_instances)]
     write_heads = read_heads = shards
     her_mode = getattr(conf, "her_mode", "final")
+    if getattr(conf, "use_prioritized_replay", False):  # prioritized replay (not a reference mode): a priority per window start
+        if conf.use_HER and her_mode == "vmap":
+            raise NotImplementedError("use_prioritized_replay is not supported with her_mode='vmap'")
+        for r in shards:
+            r.enable_priorities(alpha=getattr(conf, "per_alpha", 0.6), eps=getattr(conf, "per_eps", 1e-6), eta=getattr(conf, "per_eta", 0.9))
     if conf.use_nStep_lowerbounds:
         if her_mode == "vmap":  # Replay/__init__.py:21-23; quirk Q7 is opt-in (conf.vmap_reference_done_quirk)
             write_heads = [wrappers.NStepReturnVmap(r, conf.nStep_return_steps, conf.gamma,

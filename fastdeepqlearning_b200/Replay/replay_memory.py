@@ -80,6 +80,9 @@ class ReplayMemory:
         self.device_counter = False  # True: the draw counter lives in device memory (CUDA-graph capture of the learner step)
         self._published_len = -1     # ring length last stored next to the device-side draw counter (see publish_len)
         self._out_cache: T.Dict[tuple, dict] = {}
+        self._per_conf = None  # (alpha, eps, eta) of the priority store once enable_priorities() was called
+        self._per = None       # fdql_per handle (created with the arena)
+        self._per_beta = None  # device float32 [1]: the importance-sampling exponent the PER sampler reads at kernel time
 
     # ------------------------------------------------------------------ allocation (replay_memory.py:23-35)
     def _jit_initialize(self, widths: T.Dict[str, int], shapes=None):
@@ -105,6 +108,8 @@ class ReplayMemory:
         self._stage = [torch.zeros((self._stage_rows, self._row_floats), dtype=torch.float32).pin_memory() for _ in range(2)]
         self._stage_np = [{k: blk.numpy()[:, o:o + w] for k, o, w in zip(self._keys, self._key_off, self._widths)} for blk in self._stage]
         self._scalar_key = {k: (w == 1) for k, w in zip(self._keys, self._widths)}
+        if self._per_conf is not None:
+            self._create_per()
 
     def enable_squash_rewards(self, on=True):
         """wrappers.SquashRewards: Pohlen transform (squash_rewards.py:5-7) of the reward column of every row appended from now on."""
@@ -345,6 +350,116 @@ class ReplayMemory:
         """quirk Q3: the oldest row of an episode longer than n_step, stored once more with the n-step-truncated return."""
         check(self._lib.fdql_q3_duplicate(self._h, int(src_row), int(n_step), int(dst_row), float(gamma), _stream_ptr(self.device)))
 
+    # ------------------------------------------------------------------ prioritized replay (fdql_per_*, include/fdql.h): proportional PER
+    # (Schaul et al. 2016) over the window starts.  Not a reference mode: franQ samples uniformly (replay_memory.py:59).
+    def enable_priorities(self, alpha=0.6, eps=1e-6, eta=0.9):
+        """Keep a priority per window start: `temporal_sample(prioritized=True)` draws starts with probability q / sum(q),
+        q = (delta + eps)^alpha, and `update_priorities` sets delta from the critic's per-transition loss (eta max + (1 - eta) mean
+        over the window, R2D2's mix).  New rows enter with the largest priority written so far.  The store is created with the arena."""
+        alpha, eps, eta = float(alpha), float(eps), float(eta)
+        if not (alpha >= 0 and eps > 0 and 0 <= eta <= 1):
+            raise ValueError(f"need alpha >= 0, eps > 0, eta in [0, 1]; got alpha={alpha} eps={eps} eta={eta}")
+        if self._per is not None:
+            raise RuntimeError("priorities are already enabled")
+        self._per_conf = (alpha, eps, eta)
+        if self._h is not None:
+            self._create_per()
+
+    def _create_per(self):
+        h = C.c_void_p()
+        check(self._lib.fdql_per_create(self._h, self._temporal_len, *self._per_conf, C.byref(h)))
+        self._per = h
+        self._per_beta = torch.full((1,), 0.4, dtype=torch.float32, device=self.device)
+
+    def _require_per(self):
+        if self._per is None:
+            raise RuntimeError("prioritized sampling needs enable_priorities() and at least one stored row")
+
+    @_locked
+    def set_priority_beta(self, beta):
+        """Store the importance-sampling exponent in the device scalar the sampler reads (stream-ordered: a captured step picks it up
+        at its next replay)."""
+        self._require_per()
+        self._per_beta.fill_(float(beta))
+
+    @_locked
+    def draw_prioritized(self, n=None, beta=None, goal_mode=None, relabel_prob=0.0, xi=None):
+        """(starts, flags, goal_rows, is_weight) of n windows drawn by priority.  `xi` (device float64 [n] in [0, 1)) injects the
+        stratum offsets instead of drawing them; `beta` (None: the stored one) sets the importance-sampling exponent first."""
+        self._require_per()
+        self.flush()
+        n = self._batch_size if n is None else int(n)
+        if beta is not None:
+            self._per_beta.fill_(float(beta))
+        starts = torch.empty(n, dtype=torch.int64, device=self.device)
+        weight = torch.empty(n, dtype=torch.float32, device=self.device)
+        flags = goals = None
+        if relabel_prob > 0:
+            flags = torch.empty(n, dtype=torch.uint8, device=self.device)
+            goals = torch.empty(n, dtype=torch.int64, device=self.device)
+        if xi is not None:
+            xi = torch.as_tensor(xi, dtype=torch.float64).to(self.device).contiguous()
+            if xi.numel() != n:
+                raise ValueError(f"xi must hold {n} values")
+        if self._rng_counter_dev is None:
+            self._rng_counter_dev = torch.zeros(4, dtype=torch.int64, device=self.device)
+        ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+        check(self._lib.fdql_per_sample(self._per, n, L.GOAL_FUTURE if goal_mode is None else int(goal_mode), float(relabel_prob),
+                                        self._rng_seed, self._rng_counter, ptr(self._rng_counter_dev) if self.device_counter else None,
+                                        ptr(xi), ptr(self._per_beta), ptr(starts), ptr(flags), ptr(goals), ptr(weight),
+                                        _stream_ptr(self.device)))
+        if not self.device_counter:
+            self._rng_counter += 1
+        return starts, flags, goals, weight
+
+    @_locked
+    def update_priorities(self, starts, loss, contig=None):
+        """New priorities of the windows `starts` [B] from the per-transition loss [T-1, B(, 1)] of their transitions and the gather's
+        is_contiguous [T-1, B(, 1)] (None: all count).  Stream-ordered; duplicate starts: the last window of the batch wins."""
+        self._require_per()
+        starts = self._to_dev_i64(starts)
+        n = starts.numel()
+        loss = loss.detach().to(device=self.device, dtype=torch.float32).reshape(-1, n).contiguous()
+        if loss.shape[0] != self._temporal_len - 1:
+            raise ValueError(f"loss must be [T-1={self._temporal_len - 1}, {n}], got {tuple(loss.shape)}")
+        if contig is not None:
+            contig = contig.detach().to(device=self.device, dtype=torch.float32).reshape(loss.shape).contiguous()
+        check(self._lib.fdql_per_update(self._per, n, C.c_void_p(starts.data_ptr()), C.c_void_p(loss.data_ptr()),
+                                        C.c_void_p(contig.data_ptr()) if contig is not None else None, _stream_ptr(self.device)))
+
+    @_locked
+    def apply_pending_priorities(self):
+        """Give the rows written since the last PER call their priority (q_max, or 0 past the start range) on the current stream."""
+        if self._per is None:
+            return
+        self.flush()
+        check(self._lib.fdql_per_apply_pending(self._per, _stream_ptr(self.device)))
+
+    def priority_views(self):
+        """(leaves [maxlen], q_max [1]): zero-copy float32 views of the priority store (write leaves, then rebuild_priorities())."""
+        self._require_per()
+        leaves, qmax = C.c_void_p(), C.c_void_p()
+        check(self._lib.fdql_per_view(self._per, C.byref(leaves), C.byref(qmax)))
+        return (torch.as_tensor(_DevView(leaves.value, (self._maxlen,), (4,)), device=self.device),
+                torch.as_tensor(_DevView(qmax.value, (2,), (4,)), device=self.device)[:1])
+
+    def priority_tree(self):
+        """[(sums float64 [n_l], mins float32 [n_l]) for l = 1 .. L]: zero-copy views of the tree levels above the leaves (root last)."""
+        self._require_per()
+        out, level = [], 1
+        while True:
+            sums, mins, n = C.c_void_p(), C.c_void_p(), C.c_int64()
+            if self._lib.fdql_per_level_view(self._per, level, C.byref(sums), C.byref(mins), C.byref(n)) != L.FDQL_OK:
+                return out
+            s = torch.as_tensor(_DevView(sums.value, (n.value, 2), (8, 4)), device=self.device).view(torch.float64).reshape(-1)
+            out.append((s, torch.as_tensor(_DevView(mins.value, (n.value,), (4,)), device=self.device)))
+            level += 1
+
+    @_locked
+    def rebuild_priorities(self):
+        self._require_per()
+        check(self._lib.fdql_per_rebuild(self._per, _stream_ptr(self.device)))
+
     # ------------------------------------------------------------------ snapshot / restore (the reference never persists its replay;
     # its dormant analogue is memmap_replay_memory.py).  Every slab is saved raw -- user keys, episode extents, scan and link
     # records -- so the restored ring answers any call bit for bit, stale (partly overwritten) episodes included.
@@ -363,7 +478,15 @@ class ReplayMemory:
                 "top": self._top, "len": self._curr_len, "gamma": self.gamma, "link": (gam.value, st.value),
                 "reward_op": None if self.reward_op is None else (self.reward_op.op, list(self.reward_op.params or [])),
                 "memory": {k: v.cpu().clone() for k, v in self.memory.items()}, "ep_start": es.cpu().clone(), "ep_end": ee.cpu().clone(),
-                "scan": self._meta_rows(2).view(torch.int32).cpu().clone(), "links": self._meta_rows(3).view(torch.int32).cpu().clone()}
+                "scan": self._meta_rows(2).view(torch.int32).cpu().clone(), "links": self._meta_rows(3).view(torch.int32).cpu().clone(),
+                "per": self._per_state()}
+
+    def _per_state(self):
+        if self._per is None:
+            return None
+        self.apply_pending_priorities()
+        leaves, qmax = self.priority_views()
+        return {"conf": list(self._per_conf), "leaves": leaves.cpu().clone(), "q_max": qmax.cpu().clone()}
 
     @_locked
     def load_state_dict(self, sd):
@@ -387,6 +510,17 @@ class ReplayMemory:
         self._meta_rows(3).view(torch.int32).copy_(sd["links"].to(self.device))
         gam, st = C.c_double(float(sd["link"][0])), C.c_int32(int(sd["link"][1]))
         check(self._lib.fdql_arena_link_state(self._h, 1, C.byref(gam), C.byref(st)))
+        per = sd.get("per")
+        if per is not None and self._per is None:
+            self._per_conf = tuple(float(x) for x in per["conf"])
+            self._create_per()
+        if self._per is not None:
+            self.apply_pending_priorities()  # the restored rows were recorded as written: settle that first, then overwrite the leaves
+            if per is not None:
+                leaves, qmax = self.priority_views()
+                leaves.copy_(per["leaves"].to(self.device))
+                qmax.copy_(per["q_max"].to(self.device))
+                self.rebuild_priorities()
         torch.cuda.current_stream(self.device).synchronize()
 
     # ------------------------------------------------------------------ read side (replay_memory.py:48-70)
@@ -489,7 +623,9 @@ class ReplayMemory:
         assert (top.value, ln.value) == (self._top, self._curr_len), "host and arena cursors diverged"
 
     @_locked
-    def sample(self, idx=None) -> T.Dict[str, torch.Tensor]:
+    def sample(self, idx=None, prioritized=False) -> T.Dict[str, torch.Tensor]:
+        if prioritized:
+            raise NotImplementedError("prioritized replay draws window starts: use temporal_sample(prioritized=True)")
         if len(self) < self._batch_size:
             raise OversampleError("Trying to sample more memories than available!")
         if idx is None:
@@ -498,10 +634,26 @@ class ReplayMemory:
 
     @_locked
     def temporal_sample(self, starts=None, flags=None, goal_rows=None, exact_episode_step=False, aux=False,
-                        reuse_outputs=False, n=None, relabel_prob=0.0, goal_mode=None, length=None, exclude_keys=()):
+                        reuse_outputs=False, n=None, relabel_prob=0.0, goal_mode=None, length=None, exclude_keys=(),
+                        prioritized=False, beta=None, xi=None):
         """[T, B, w] window gather (replay_memory.py:54-66).  `starts` (and for hindsight relabelling `flags`,
         `goal_rows`) inject the index streams; when absent they are drawn on the device.  With `aux=True` the dict
-        also carries `mask`, `is_contiguous` and `loss_weight` (deepQlearning.py:201-203,222-225)."""
+        also carries `mask`, `is_contiguous` and `loss_weight` (deepQlearning.py:201-203,222-225).
+        `prioritized=True` (after enable_priorities) draws the starts by priority (draw_prioritized: `beta`, `xi`) and gathers them
+        with the same kernel as injected starts; the dict then also carries `is_weight` [B] and the `starts` [B] drawn."""
+        if prioritized:
+            if starts is not None or length is not None:
+                raise ValueError("prioritized sampling draws its own starts")
+            if len(self) < self._temporal_len * 2 or len(self) < self._batch_size:
+                raise OversampleError("Trying to sample more memories than available!")
+            starts, flags, goal_rows, weight = self.draw_prioritized(n, beta, goal_mode, relabel_prob, xi)
+            # every drawn start is < len - T, so its window never wraps: the capacity as modulus gives the rows len would, and stays
+            # right inside a captured step while the ring grows
+            res = self.temporal_sample(starts=starts, flags=flags, goal_rows=goal_rows, exact_episode_step=exact_episode_step, aux=aux,
+                                       reuse_outputs=reuse_outputs, length=self._maxlen, exclude_keys=exclude_keys)
+            self.last_streams = (starts, flags, goal_rows)
+            res["is_weight"], res["starts"] = weight, starts
+            return res
         _len = len(self) if length is None else int(length)
         Tn = self._temporal_len
         n = self._batch_size if n is None else int(n)
@@ -573,6 +725,12 @@ class ReplayMemory:
         return self.temporal_sample(starts=batch, length=_len)
 
     def __del__(self):
+        per, self._per = getattr(self, "_per", None), None
+        if per is not None:
+            try:
+                self._lib.fdql_per_destroy(per)  # before its arena
+            except Exception:
+                pass
         h, self._h = getattr(self, "_h", None), None
         if h is not None:
             try:

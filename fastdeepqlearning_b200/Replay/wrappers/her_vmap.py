@@ -62,6 +62,8 @@ class HindsightVmapRead(ReplayMemoryWrapper):
         self.aux = aux
 
     def temporal_sample(self, column=None, **kwargs):
+        if kwargs.pop("prioritized", False):
+            raise NotImplementedError("prioritized replay is not supported with the vmap hindsight variant")
         ring = self.replay_buffer
         while hasattr(ring, "replay_buffer") or hasattr(ring, "replay"):
             ring = getattr(ring, "replay_buffer", None) or ring.replay

@@ -78,6 +78,14 @@ _SIGNATURES = {
     "fdql_sac_min_target_loss_dev_alpha": (C.c_int, [_i64, _i32, _p, _p, _p, _p, _p, _p, _p, _p, _f32, _p, _p, _p, _p]),
     "fdql_hotpath_step_host": (C.c_int, [_p, _i64, _i32, _i64, _p, _p, _p, _i32, C.POINTER(_f32), _i32, _f64, _u32, _pp,
                                          _i32, _i32, _p, _p, _p, _f32, _p, _p, _p]),
+    "fdql_per_create": (C.c_int, [_p, _i32, _f32, _f32, _f32, C.POINTER(_p)]),
+    "fdql_per_destroy": (C.c_int, [_p]),
+    "fdql_per_sample": (C.c_int, [_p, _i64, _i32, _f32, _u64, _u64, _p, _p, _p, _p, _p, _p, _p, _p]),
+    "fdql_per_update": (C.c_int, [_p, _i64, _p, _p, _p, _p]),
+    "fdql_per_apply_pending": (C.c_int, [_p, _p]),
+    "fdql_per_view": (C.c_int, [_p, C.POINTER(_p), C.POINTER(_p)]),
+    "fdql_per_level_view": (C.c_int, [_p, _i32, C.POINTER(_p), C.POINTER(_p), C.POINTER(_i64)]),
+    "fdql_per_rebuild": (C.c_int, [_p, _p]),
 }
 EXPORTS = tuple(_SIGNATURES)
 

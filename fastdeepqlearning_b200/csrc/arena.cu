@@ -372,7 +372,37 @@ int flush_pending_invalidation(const Arena* ca, cudaStream_t st) {
   return FDQL_OK;
 }
 
+std::mutex& cursor_mutex() {
+  static std::mutex m;
+  return m;
+}
+
+// rows [first, first + n) (mod capacity) were (over)written: their leaves of the priority store become q_max or 0 (per.cu).
+// Consecutive writes coalesce into one interval; when the short list is full its last entry grows to the whole ring.
+static void note_per_rows(Arena* a, int64_t first, int64_t n) {
+  const int64_t cap = a->dev.capacity;
+  if (a->per == nullptr || n <= 0) return;
+  if (n > cap) n = cap;
+  if (a->n_per_pending > 0) {
+    int64_t* last = a->per_pending[a->n_per_pending - 1];
+    if ((last[0] + last[1]) % cap == first) {
+      last[1] = last[1] + n > cap ? cap : last[1] + n;
+      return;
+    }
+    if (a->n_per_pending == 4) {
+      last[0] = 0;
+      last[1] = cap;
+      return;
+    }
+  }
+  a->per_pending[a->n_per_pending][0] = first;
+  a->per_pending[a->n_per_pending][1] = n;
+  ++a->n_per_pending;
+}
+
 static void advance_cursor(Arena* a, int64_t n) {
+  std::lock_guard<std::mutex> lk(cursor_mutex());
+  note_per_rows(a, a->top, n);
   const int64_t cap = a->dev.capacity, top = a->top;
   int64_t mx;
   if (n >= cap) mx = cap - 1;
@@ -521,6 +551,7 @@ int fdql_arena_info(const fdql_arena* a, int64_t* capacity, int64_t* top, int64_
 int fdql_arena_set_cursor(fdql_arena* a, int64_t top, int64_t len) {
   FDQL_REQUIRE(a != nullptr, "null arena");
   FDQL_REQUIRE(top >= 0 && top < a->dev.capacity && len >= 0 && len <= a->dev.capacity, "cursor out of range");
+  std::lock_guard<std::mutex> lk(cursor_mutex());  // a length change moves the priority store's eligible range (per.cu)
   a->top = top;
   a->len = len;
   a->pending_inval_row = -1;

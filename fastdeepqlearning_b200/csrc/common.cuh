@@ -5,6 +5,8 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <mutex>
+
 #include "../../include/fdql.h"
 
 namespace fdql {
@@ -174,9 +176,16 @@ struct Arena {
   int32_t append_src_stride, append_squash;  // set around fdql_arena_append by the packed host form (see arena.cu)
   int64_t rows_written;        // rows [0, rows_written) of the ring have held data (capacity once it has wrapped)
   int64_t pending_inval_row;   // first row behind the write head whose episode may have lost its beginning (-1: none); see arena.cu
+  // prioritized replay (per.cu): the arena's priority store, if one was created, and the ring intervals {first row, rows} written since
+  // its last activation pass.  Writers only record them here (under cursor_mutex()); the PER calls apply them on their own stream.
+  ::fdql_per* per;
+  int64_t per_pending[4][2];
+  int32_t n_per_pending;
 };
 
 int flush_pending_invalidation(const Arena* a, cudaStream_t st);
+// serialises the host cursor (top, len) and the pending priority intervals between a writer thread and the PER calls of a reader
+std::mutex& cursor_mutex();
 
 int upload_reward_spec(const Arena* a, int32_t op, const float* params_host, int32_t n_params, cudaStream_t st,
                        RewardSpec* out);

@@ -12,29 +12,11 @@
 #include "common.cuh"
 #include "goal_eval.cuh"
 #include "tqc_group.cuh"
+#include "draw.cuh"
 
 #include <atomic>
 
 namespace fdql {
-
-// ---- counter-based generator (Philox4x32-10) ----------------------------------------------------
-__device__ __forceinline__ void philox_round(uint32_t& c0, uint32_t& c1, uint32_t& c2, uint32_t& c3, uint32_t k0, uint32_t k1) {
-  const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
-  const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
-  const uint32_t n0 = hi1 ^ c1 ^ k0, n2 = hi0 ^ c3 ^ k1;
-  c0 = n0; c1 = lo1; c2 = n2; c3 = lo0;
-}
-__device__ __forceinline__ uint4 philox4x32(uint64_t ctr_lo, uint64_t ctr_hi, uint64_t key) {
-  uint32_t c0 = (uint32_t)ctr_lo, c1 = (uint32_t)(ctr_lo >> 32), c2 = (uint32_t)ctr_hi, c3 = (uint32_t)(ctr_hi >> 32);
-  uint32_t k0 = (uint32_t)key, k1 = (uint32_t)(key >> 32);
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    philox_round(c0, c1, c2, c3, k0, k1);
-    k0 += 0x9E3779B9u;
-    k1 += 0xBB67AE85u;
-  }
-  return make_uint4(c0, c1, c2, c3);
-}
 
 // a whole 8-float scalar record (one 32-byte sector) in ONE load instruction: a thread-per-window phase reads records of 32
 // unrelated rows per warp instruction, so every separate column load costs the L1 another 32 sector look-ups
@@ -75,19 +57,7 @@ __device__ __forceinline__ void draw_window(const ArenaDev& A, int64_t b, int64_
     es = __float_as_int(__ldg(rec + A.col_ep_start));
     ee = __float_as_int(__ldg(rec + A.col_ep_end));
   }
-  f = (es >= 0) && ((float)x.z * 2.3283064365386963e-10f < relabel_prob);
-  if (f) {
-    const int64_t cap = A.capacity;
-    if (goal_mode == FDQL_GOAL_FINAL) {
-      g = ee;
-    } else if (goal_mode == FDQL_GOAL_RANDOM) {
-      const int64_t L = (ee - es + (ee < es ? cap : 0)) + 1;
-      g = ring_row(es, (int64_t)__umulhi(x.w, (uint32_t)L), cap);
-    } else {  // FUTURE: a row strictly after the start row, the last row when there is none
-      const int64_t m = ee - s + (ee < s ? cap : 0);
-      g = m == 0 ? ee : ring_row(s, 1 + (int64_t)__umulhi(x.w, (uint32_t)m), cap);
-    }
-  }
+  hindsight_pick(A.capacity, s, es, ee, x.z, x.w, goal_mode, relabel_prob, f, g);
 }
 // counter_dev[2] (optional, non-zero): the ring's current length, so that a captured launch keeps sampling the whole ring while it
 // fills (the range len - T is otherwise baked into the launch)
@@ -96,34 +66,6 @@ __device__ __forceinline__ int64_t device_draw_range(const unsigned long long* c
   const unsigned long long len = *reinterpret_cast<const volatile unsigned long long*>(counter_dev + 2);
   return len != 0ull ? (int64_t)len - T : range;
 }
-// counter_dev (optional): {draw counter, block ticket} in device memory, so that a captured CUDA graph draws fresh streams at
-// every replay.  Every block reads the counter before it takes its ticket; the block with the last ticket advances it.
-// (role form: `tid` = thread index within the role, `n_blk` = blocks that take a ticket, `bar_id` / `n_threads` = the role's barrier,
-// see role_barrier in tqc_group.cuh; the defaults are "the whole block of an ordinary launch")
-__device__ __forceinline__ uint64_t device_draw_counter(unsigned long long* counter_dev, uint64_t counter, int tid = -1, int n_blk = 0,
-                                                        int bar_id = 0, int n_threads = 0) {
-  __shared__ unsigned long long sh_ctr;
-  if (counter_dev == nullptr) return counter;
-  if (tid < 0) {
-    tid = (int)threadIdx.x;
-    n_blk = (int)gridDim.x;
-  }
-  if (tid == 0) sh_ctr = *reinterpret_cast<volatile unsigned long long*>(counter_dev);
-  role_barrier(bar_id, n_threads);
-  counter += sh_ctr;
-  role_barrier(bar_id, n_threads);
-  if (tid == 0) {
-    __threadfence();
-    const unsigned long long ticket = atomicAdd(counter_dev + 1, 1ull);
-    if (ticket == (unsigned long long)n_blk - 1) {
-      counter_dev[1] = 0ull;
-      counter_dev[0] = sh_ctr + 1ull;
-      __threadfence();
-    }
-  }
-  return counter;
-}
-
 // starts ~ U[0, len-T) like np.random.randint(0, len-T, B) (replay_memory.py:59); flag ~ Bernoulli(p); goal row by mode
 // over the committed extents of the start row's episode (her.py:48-53).  Uncommitted rows are never relabelled.
 __global__ void __launch_bounds__(256)

@@ -285,6 +285,54 @@ int fdql_hotpath_step_host(fdql_arena* a, int64_t n_windows, int32_t T, int64_t 
                            const float* q_pred_host, const float* next_log_pi_host, float alpha, float* loss_host,
                            float* grad_q_host, void* stream);
 
+/* ---- prioritized experience replay: proportional PER with importance-sampling correction (Schaul, Quan, Antonoglou, Silver,
+ *      "Prioritized Experience Replay", ICLR 2016).  NOT a reference mode: franQ draws every window start uniformly
+ *      (replay_memory.py:59); this is an opt-in extension like FDQL_GOAL_FUTURE.
+ *
+ * A priority store belongs to one arena (at most one per arena; destroy it before the arena) and to one window length T.  It holds a
+ * leaf q[r] = p_r^alpha (fp32) per ring row r, taken as a window start, under a 32-ary tree of fp64 sums and fp32 minima (4 + ~4/31 x
+ * 12 bytes per row, plus a 4-byte claim slot per row for duplicate starts of an update: ~8.5 bytes per row, 85 MB at 1e7 rows).
+ * Every node is recomputed from its children in one fixed order, never adjusted by atomics: the same call sequence gives the same tree
+ * bits whatever the scheduling.
+ *
+ * Eligibility invariant: q[r] > 0 iff r < len - T, the start range of quirk Q2 (np.random.randint(0, len - T)).  A row gets q_max
+ * (a device scalar: the running max of every leaf written, 1.0 at creation) when it is (over)written, or when it becomes eligible
+ * because len grew.  The writers (fdql_arena_append and its host forms, fdql_arena_reserve and so fdql_her_flush_episodes /
+ * fdql_q3_duplicate / vmap rows, fdql_arena_set_cursor) run on the writer's stream and only RECORD the rows they wrote on the host
+ * side of the arena; every tree write happens on the stream of the PER calls (the reader's): the next fdql_per_sample or
+ * fdql_per_update, or fdql_per_apply_pending, applies what was recorded.  While `stream` is being captured into a CUDA graph the
+ * recorded rows are left for the next uncaptured call (a captured copy would re-apply them at every replay). */
+typedef struct fdql_per fdql_per;
+
+/* alpha >= 0 (priority exponent), eps > 0 (added to every |delta|), eta in [0, 1] (R2D2's max / mean mix over a window), T >= 2.
+ * Rows already in the ring are activated at once. */
+int fdql_per_create(fdql_arena* a, int32_t T, float alpha, float eps, float eta, fdql_per** out);
+int fdql_per_destroy(fdql_per* per);
+/* n windows drawn by priority, stratified: window b takes the target S (b + xi_b) / n, S the root sum, and descends to the leaf whose
+ * prefix interval holds it (fp rounding past the last positive leaf is clamped to that leaf).  xi_b comes from Philox (b, counter, seed)
+ * with the counter / counter_dev protocol of fdql_sample_streams (counter_dev[2] is not read: the tree holds the eligible range), or from
+ * xi (device double[n] in [0, 1), may be NULL) for parity runs.  flags / goal_rows (may be NULL) follow fdql_sample_streams' hindsight
+ * rules for the drawn start.  is_weight (may be NULL) [n] = (q_min / q[start])^beta with q_min the smallest positive leaf (Schaul's
+ * (N P)^-beta / max w) and beta read from beta_dev[0] at kernel time (an annealed beta inside a captured graph).
+ * FDQL_EOVERSAMPLE when len < 2T (under the invariant also the only case of S == 0). */
+int fdql_per_sample(fdql_per* per, int64_t n, int32_t goal_mode, float relabel_prob, uint64_t seed, uint64_t counter,
+                    uint64_t* counter_dev, const double* xi, const float* beta_dev, int64_t* starts, uint8_t* flags,
+                    int64_t* goal_rows, float* is_weight, void* stream);
+/* new priorities of n windows from the per-transition loss [T-1, n] of their transitions (a loss kernel's `loss`, m = t n + b) and the
+ * gather's is_contiguous [T-1, n] (NULL: every transition counts): delta_b = eta max_t + (1 - eta) mean_t over the contiguous ones
+ * (0 when none), q = (delta_b + eps)^alpha.  A non-finite loss or q writes q_max instead.  Duplicate starts: the largest b wins.
+ * Leaves that are 0 (rows that are not eligible starts) stay 0. */
+int fdql_per_update(fdql_per* per, int64_t n, const int64_t* starts, const float* loss, const float* contig, void* stream);
+int fdql_per_apply_pending(fdql_per* per, void* stream);
+/* the leaves [capacity] and q_max_dev[0] (device memory) for snapshots and tests; after writing leaves call fdql_per_rebuild */
+int fdql_per_view(const fdql_per* per, float** leaves, float** q_max_dev);
+/* node arrays of tree level `level` in [1, L] (level L is the root): fp64 sums and fp32 minima of positive leaves (+inf: none), n_nodes
+ * of them; node i covers entries 32 i .. 32 i + 31 of the level below (level 0: the leaves).  A level past L fails with L in the
+ * message.  For tests and tools. */
+int fdql_per_level_view(const fdql_per* per, int32_t level, double** sums, float** mins, int64_t* n_nodes);
+/* every node of the tree from the leaves */
+int fdql_per_rebuild(fdql_per* per, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
