@@ -86,6 +86,9 @@ _SIGNATURES = {
     "fdql_per_view": (C.c_int, [_p, C.POINTER(_p), C.POINTER(_p)]),
     "fdql_per_level_view": (C.c_int, [_p, _i32, C.POINTER(_p), C.POINTER(_p), C.POINTER(_i64)]),
     "fdql_per_rebuild": (C.c_int, [_p, _p]),
+    "fdql_fused_pass_per": (C.c_int, [_p, _i64, _i32, _f32, _u64, _u64, _p, _p, _p, _p, _p, _p, _p, _p, _i32, C.POINTER(_f32), _i32, _f64,
+                                      _u32, _i32, _pp, _p, _p, _p, _i64, _i32, _i32, _p, _p, _p, _p, _p, _p, _p, _f32, _f32, _p, _p, _p,
+                                      _p, _p, _p]),
 }
 EXPORTS = tuple(_SIGNATURES)
 

@@ -208,6 +208,9 @@ struct DrawSpec {
   // kernel together with this loss (a TqcArgs of tqc_group.cuh) and *fused is set to 1; otherwise the gather launches alone
   const void* fuse_tqc = nullptr;
   int* fused = nullptr;
+  // prioritized fused pass (fdql_fused_pass_per): the starts come from this priority tree (a PerDraw of draw.cuh); only the fused
+  // kernel draws them -- any shape it does not serve returns 1 with nothing launched
+  const void* per = nullptr;
 };
 // returns FDQL_OK, an error, or (with draw != nullptr) 1 when this shape is not served by the fused kernel (nothing launched)
 int launch_gather(const fdql_arena* a, int64_t n, int64_t b_begin, int64_t b_end, int32_t T, int64_t len, const int64_t* starts,

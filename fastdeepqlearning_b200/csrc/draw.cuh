@@ -43,6 +43,64 @@ __device__ __forceinline__ void hindsight_pick(int64_t cap, int64_t s, int es, i
   }
 }
 
+// ---- prioritized draw (per.cu; the gather role of fdql_fused_pass_per in sample.cu) --------------
+constexpr int kPerMaxLevels = 8;  // 32^7 > 2^31 > capacity
+
+// device view of a priority store (see per.cu): leaves [n[0]] under levels 1..n_levels of fp64 sums / fp32 minima
+struct PerDev {
+  int32_t n_levels;
+  int64_t n[kPerMaxLevels];
+  float* leaves;
+  int32_t* owner;
+  double* sums[kPerMaxLevels];
+  float* mins[kPerMaxLevels];
+  float* q_max;
+};
+
+// what the gather role of a prioritized fused pass needs besides GatherArgs
+struct PerDraw {
+  PerDev P;
+  const double* xi;       // injected offsets or NULL (Philox)
+  const float* beta_dev;  // importance-weight exponent, read at kernel time
+  float* is_weight;       // [n] or NULL
+  float* critic_weight;   // [T-1, n] = aux_weight * is_weight, or NULL
+};
+
+// xi_b from the first two Philox words: 53 random bits in [0, 1)
+__device__ __forceinline__ double per_uniform(const uint4& x) { return (double)((((uint64_t)x.x << 32) | x.y) >> 11) * 0x1.0p-53; }
+// stratified target of window b of n: S (b + xi_b) / n
+__device__ __forceinline__ double per_target(double S, int64_t b, int64_t n, double u) { return S * (((double)b + u) / (double)n); }
+// (q_min / q[s])^beta in fp64, stored as fp32
+__device__ __forceinline__ float per_is_weight(float qmin, float q, float beta) { return (float)pow((double)qmin / (double)q, (double)beta); }
+
+// One level of the descent of ONE window by one warp, in two steps so that children shared by many windows are scanned once.
+// per_scan: inclusive / exclusive prefix sums of the 32 children (`v` = this lane's child, 0 past the level's end) in Kogge-Stone
+// order.  That order is part of the draw: every prioritized sampler descends through these two functions, so they give the same bits.
+__device__ __forceinline__ void per_scan(double v, int lane, double& incl, double& excl) {
+  incl = v;
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    const double o = shfl_up_f64(incl, d);
+    if (lane >= d) incl += o;
+  }
+  excl = shfl_up_f64(incl, 1);
+  if (lane == 0) excl = 0.0;
+}
+// per_pick: the first child whose inclusive prefix exceeds the window's remaining target t (warp-uniform), or the last positive
+// child when fp rounding put t past it; t loses the sum of the children before the pick.
+__device__ __forceinline__ int per_pick(double v, double incl, double excl, double& t) {
+  const unsigned hit = __ballot_sync(kFull, incl > t);
+  int pick;
+  if (hit) {
+    pick = __ffs(hit) - 1;
+  } else {  // fp rounding put the target past the last positive child: clamp to it
+    const unsigned pos = __ballot_sync(kFull, v > 0.0);
+    pick = pos ? 31 - __clz(pos) : 0;
+  }
+  t -= shfl_idx_f64(excl, pick);
+  return pick;
+}
+
 // counter_dev (optional): {draw counter, block ticket} in device memory, so that a captured CUDA graph draws fresh streams at
 // every replay.  Every block reads the counter before it takes its ticket; the block with the last ticket advances it.
 // (role form: `tid` = thread index within the role, `n_blk` = blocks that take a ticket, `bar_id` / `n_threads` = the role's barrier,

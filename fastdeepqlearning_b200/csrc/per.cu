@@ -12,7 +12,7 @@
 #include "common.cuh"
 #include "draw.cuh"
 
-constexpr int kPerMaxLevels = 8;  // 32^7 > 2^31 > capacity
+using fdql::kPerMaxLevels;
 
 struct fdql_per {
   fdql_arena* a;
@@ -29,16 +29,6 @@ struct fdql_per {
 };
 
 namespace fdql {
-
-struct PerDev {
-  int32_t n_levels;
-  int64_t n[kPerMaxLevels];
-  float* leaves;
-  int32_t* owner;
-  double* sums[kPerMaxLevels];
-  float* mins[kPerMaxLevels];
-  float* q_max;
-};
 
 static PerDev per_dev(const fdql_per* p) {
   PerDev d;
@@ -126,6 +116,15 @@ __global__ void __launch_bounds__(256) per_update_level_kernel(PerDev P, int l, 
   if (l == 1 && lane_id() == 0) P.owner[s] = -1;
 }
 
+// what level 1 of per_update_level_kernel does besides the node when level 1 is rebuilt whole: hand the owner slots back, fold q_max
+__global__ void __launch_bounds__(256) per_release_kernel(PerDev P, int64_t n, const int64_t* __restrict__ starts) {
+  const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (b == 0) P.q_max[0] = fmaxf(P.q_max[0], P.q_max[1]);
+  if (b >= n) return;
+  const int64_t s = starts[b];
+  if (s >= 0 && s < P.n[0]) P.owner[s] = -1;
+}
+
 // duplicate starts in one batch: the largest window index wins
 __global__ void __launch_bounds__(256) per_claim_kernel(PerDev P, int64_t n, const int64_t* __restrict__ starts) {
   const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -178,39 +177,20 @@ per_sample_kernel(PerDev P, ArenaDev A, int64_t n, int goal_mode, float relabel_
   const int L = P.n_levels;
   uint4 x = make_uint4(0u, 0u, 0u, 0u);
   if (xi == nullptr || flags != nullptr) x = philox4x32((uint64_t)b, counter, seed);
-  const double u = xi != nullptr ? xi[b] : (double)((((uint64_t)x.x << 32) | x.y) >> 11) * 0x1.0p-53;
-  const double S = P.sums[L][0];
-  double t = S * (((double)b + u) / (double)n);
+  const double u = xi != nullptr ? xi[b] : per_uniform(x);
+  double t = per_target(P.sums[L][0], b, n, u);
   int64_t node = 0;
   for (int l = L; l >= 1; --l) {
     const int64_t c = 32 * node + lane;
     double v = 0.0;
     if (c < P.n[l - 1]) v = l == 1 ? (double)P.leaves[c] : P.sums[l - 1][c];
-    double incl = v;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      const double o = shfl_up_f64(incl, d);
-      if (lane >= d) incl += o;
-    }
-    double excl = shfl_up_f64(incl, 1);
-    if (lane == 0) excl = 0.0;
-    const unsigned hit = __ballot_sync(kFull, incl > t);
-    int pick;
-    if (hit) {
-      pick = __ffs(hit) - 1;
-    } else {  // fp rounding put the target past the last positive child: clamp to it
-      const unsigned pos = __ballot_sync(kFull, v > 0.0);
-      pick = pos ? 31 - __clz(pos) : 0;
-    }
-    t -= shfl_idx_f64(excl, pick);
-    node = c - lane + pick;
+    double incl, excl;
+    per_scan(v, lane, incl, excl);
+    node = c - lane + per_pick(v, incl, excl, t);
   }
   if (lane != 0) return;
   starts[b] = node;
-  if (is_weight != nullptr) {
-    const double qmin = (double)P.mins[L][0], q = (double)P.leaves[node];
-    is_weight[b] = (float)pow(qmin / q, (double)beta_dev[0]);
-  }
+  if (is_weight != nullptr) is_weight[b] = per_is_weight(P.mins[L][0], P.leaves[node], beta_dev[0]);
   if (flags == nullptr) return;
   const float* rec = A.rec + node * (int64_t)A.rec_stride;
   const int es = __float_as_int(__ldg(rec + A.col_ep_start)), ee = __float_as_int(__ldg(rec + A.col_ep_end));
@@ -304,6 +284,38 @@ static int apply_pending(fdql_per* p, cudaStream_t st) {
   per_set_leaves_kernel<<<grid_for(total, a->num_sms), 256, 0, st>>>(per_dev(p), iv, total, len - p->T);
   FDQL_CUDA(cudaGetLastError());
   return refresh_ancestors(p, iv, st);
+}
+
+// new leaves for n windows, then their ancestors.  Level l is recomputed per window (one warp each, the same node as often as windows
+// share it) while the batch has fewer windows than the level has nodes, and whole (one warp per node) from there up: at 262144 windows
+// over 1e7 rows that is levels 2.. (9766 nodes and fewer) instead of 262144 recomputations of each.  Either form recomputes a node from
+// its children in the same order, so the tree bits do not depend on the choice, and the choice depends on n alone (capturable).
+static int launch_update(const fdql_per* p, int64_t n, const int64_t* starts, const float* loss, const float* contig, cudaStream_t st) {
+  const PerDev D = per_dev(p);
+  const unsigned g1 = (unsigned)((n + 255) / 256), gw = (unsigned)((n + 7) / 8);
+  per_claim_kernel<<<g1, 256, 0, st>>>(D, n, starts);
+  per_write_leaves_kernel<<<g1, 256, 0, st>>>(D, n, p->T - 1, starts, loss, contig, (double)p->alpha, (double)p->eps, (double)p->eta);
+  for (int l = 1; l <= p->n_levels; ++l) {
+    if (n < p->n[l]) {
+      per_update_level_kernel<<<gw, 256, 0, st>>>(D, l, n, starts);
+      continue;
+    }
+    Intervals all;
+    all.k = 1;
+    all.lo[0] = 0;
+    all.hi[0] = p->n[l];
+    per_level_kernel<<<grid_for(p->n[l] * 32, p->a->num_sms), 256, 0, st>>>(D, l, all, p->n[l]);
+    if (l == 1) per_release_kernel<<<g1, 256, 0, st>>>(D, n, starts);
+  }
+  FDQL_CUDA(cudaGetLastError());
+  return FDQL_OK;
+}
+
+// critic_weight[t, b] = aux_weight[t, b] * is_weight[b]: what the gather role of the fused kernel writes, for the separate launches
+__global__ void __launch_bounds__(256) per_critic_weight_kernel(int64_t n, int64_t total, const float* __restrict__ aux_weight,
+                                                                const float* __restrict__ is_weight, float* __restrict__ critic_weight) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < total) critic_weight[i] = aux_weight[i] * is_weight[i % n];
 }
 
 }  // namespace fdql
@@ -454,15 +466,94 @@ int fdql_per_update(fdql_per* p, int64_t n, const int64_t* starts, const float* 
   if (n == 0) return FDQL_OK;
   FDQL_REQUIRE(starts != nullptr && loss != nullptr, "null argument");
   const cudaStream_t st = (cudaStream_t)stream;
-  int rc = apply_pending(p, st);
+  const int rc = apply_pending(p, st);
   if (rc) return rc;
-  const PerDev D = per_dev(p);
-  const unsigned g1 = (unsigned)((n + 255) / 256), gw = (unsigned)((n + 7) / 8);
-  per_claim_kernel<<<g1, 256, 0, st>>>(D, n, starts);
-  per_write_leaves_kernel<<<g1, 256, 0, st>>>(D, n, p->T - 1, starts, loss, contig, (double)p->alpha, (double)p->eps, (double)p->eta);
-  for (int l = 1; l <= p->n_levels; ++l) per_update_level_kernel<<<gw, 256, 0, st>>>(D, l, n, starts);
-  FDQL_CUDA(cudaGetLastError());
-  return FDQL_OK;
+  return launch_update(p, n, starts, loss, contig, st);
+}
+
+int fdql_fused_pass_per(fdql_per* p, int64_t n_windows, int32_t goal_mode, float relabel_prob, uint64_t seed, uint64_t counter,
+                        uint64_t* counter_dev, const double* xi, const float* beta_dev, int64_t* starts, uint8_t* flags, int64_t* goal_rows,
+                        float* is_weight, float* critic_weight, int32_t reward_op, const float* reward_params_host, int32_t n_params,
+                        double gamma, uint32_t opts, int32_t batch_for_weight, float* const* out, float* aux_mask, float* aux_contig,
+                        float* aux_weight, int64_t M, int32_t n_atoms, int32_t n_drop, const float* next_z, const float* q_pred,
+                        const float* next_log_pi, const float* reward, const float* mask, const float* mc_return, const float* grad_scale,
+                        float alpha, float loss_gamma, float* loss, float* grad_q, double* stats, const int64_t* loss_starts,
+                        const float* loss_contig, void* stream) {
+  // (every check that needs no field of the store comes first)
+  FDQL_REQUIRE(p != nullptr, "null priority store");
+  FDQL_REQUIRE(n_windows >= 0 && M >= 0, "bad sizes");
+  FDQL_REQUIRE(n_windows == 0 || (starts != nullptr && out != nullptr), "null gather argument");
+  FDQL_REQUIRE((flags == nullptr) == (goal_rows == nullptr), "flags and goal_rows come together");
+  FDQL_REQUIRE(n_windows == 0 || (goal_mode >= FDQL_GOAL_FINAL && goal_mode <= FDQL_GOAL_FUTURE), "bad goal mode");
+  FDQL_REQUIRE(critic_weight == nullptr || (opts & FDQL_OPT_EMIT_LEARNER_AUX), "critic_weight needs FDQL_OPT_EMIT_LEARNER_AUX");
+  FDQL_REQUIRE(critic_weight == nullptr || (aux_weight != nullptr && is_weight != nullptr), "critic_weight needs aux_weight and is_weight");
+  FDQL_REQUIRE(is_weight == nullptr || beta_dev != nullptr, "importance weights need beta_dev");
+  if (M > 0) {
+    FDQL_REQUIRE(loss_starts != nullptr && loss != nullptr, "the loss half needs loss_starts and loss (the priority update reads them)");
+    FDQL_REQUIRE(n_atoms >= 2 && n_atoms <= 256, "n_atoms must be in [2, 256], got %d", n_atoms);
+    FDQL_REQUIRE(n_drop >= 1 && n_drop < n_atoms, "n_drop must be in [1, n_atoms); got %d", n_drop);  // quirk Q8, as fdql_tqc_loss
+    FDQL_REQUIRE(next_z && q_pred && reward && mask && grad_q, "null loss argument");
+  }
+  const int32_t T = p->T;
+  FDQL_REQUIRE(M % (T - 1) == 0, "M = %lld is not a whole number of windows of T - 1 = %d transitions", (long long)M, T - 1);
+  fdql_arena* a = p->a;
+  const cudaStream_t st = (cudaStream_t)stream;
+  int64_t len;
+  {
+    std::lock_guard<std::mutex> lk(cursor_mutex());
+    len = a->len;
+  }
+  if (n_windows > 0 && len < 2 * (int64_t)T) {  // as fdql_per_sample
+    set_error("OversampleError: ring holds %lld rows, asked for %lld windows of %d", (long long)len, (long long)n_windows, T);
+    return FDQL_EOVERSAMPLE;
+  }
+  if (n_windows > 0 && (opts & FDQL_OPT_EMIT_LEARNER_AUX))
+    FDQL_REQUIRE(a->dev.col_task_done >= 0 && a->dev.col_ep_step >= 0, "learner aux needs task_done and episode_step keys");
+  int rc = flush_pending_invalidation(a, st);
+  if (rc == FDQL_OK) rc = apply_pending(p, st);
+  if (rc) return rc;
+  TqcArgs t{M, n_atoms, n_atoms, n_drop, next_z, q_pred, next_log_pi, reward, mask, mc_return, grad_scale, alpha, loss_gamma, loss, grad_q,
+            nullptr, stats, nullptr, 0};
+  // window modulus of the gather: the capacity, not len.  Every drawn start is < len - T, so no window wraps and the rows are the same;
+  // len would be frozen into a captured launch while the tree (and so the draw) follows the ring as it grows.
+  const int64_t cap = a->dev.capacity;
+  int fused = 0;
+  if (n_windows > 0 && M > 0) {
+    PerDraw pd;
+    pd.P = per_dev(p);
+    pd.xi = xi;
+    pd.beta_dev = beta_dev;
+    pd.is_weight = is_weight;
+    pd.critic_weight = critic_weight;
+    DrawSpec d{len - T, goal_mode, relabel_prob, seed, counter, reinterpret_cast<unsigned long long*>(counter_dev), starts, flags, goal_rows};
+    d.fuse_tqc = &t;
+    d.fused = &fused;
+    d.per = &pd;
+    rc = launch_gather(a, n_windows, 0, n_windows, T, cap, nullptr, nullptr, nullptr, reward_op, reward_params_host, n_params, gamma,
+                       opts | FDQL_OPT_CORESIDENT, batch_for_weight, out, aux_mask, aux_contig, aux_weight, st, &d);
+    if (rc != FDQL_OK && rc != 1) return rc;
+  }
+  if (n_windows > 0 && !fused) {
+    // the separate launches, with the same results: prioritized streams, the co-resident gather on them, the critic weights
+    rc = fdql_per_sample(p, n_windows, goal_mode, relabel_prob, seed, counter, counter_dev, xi, beta_dev, starts, flags, goal_rows, is_weight,
+                         stream);
+    if (rc == FDQL_OK)
+      rc = launch_gather(a, n_windows, 0, n_windows, T, cap, starts, flags, goal_rows, reward_op, reward_params_host, n_params, gamma,
+                         opts | FDQL_OPT_CORESIDENT, batch_for_weight, out, aux_mask, aux_contig, aux_weight, st);
+    if (rc) return rc;
+    if (critic_weight != nullptr) {
+      const int64_t total = (int64_t)(T - 1) * n_windows;
+      per_critic_weight_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(n_windows, total, aux_weight, is_weight, critic_weight);
+      FDQL_CUDA(cudaGetLastError());
+    }
+  }
+  if (M == 0) return FDQL_OK;
+  if (!fused) {
+    rc = launch_tqc(t, st);
+    if (rc) return rc;
+  }
+  // after the launch that read the tree for batch k+1: the priorities of batch k
+  return launch_update(p, M / (T - 1), loss_starts, loss, loss_contig, st);
 }
 
 }  // extern "C"

@@ -36,13 +36,20 @@ __device__ __forceinline__ float pick8(const float (&r)[8], int c) {  // r[c] fo
 // (rec8: when given, the start row's scalar record is 8 floats wide and is returned whole for the caller's own use)
 // record columns of the builds specialised on a window length (window_scalar_phase, TC > 0)
 constexpr int kCanonReward = 0, kCanonTaskDone = 1, kCanonEpStep = 3, kCanonMcReturn = 4, kCanonScal = 5, kCanonEpStart = 5, kCanonEpEnd = 6;
-template <int TC = 0>
+// (PER: the start was drawn from the priority tree, per_descend_chunk; per_z / per_w are the last two words of the window's Philox draw)
+template <int TC = 0, bool PER = false>
 __device__ __forceinline__ void draw_window(const ArenaDev& A, int64_t b, int64_t range, int goal_mode, float relabel_prob, uint64_t seed,
                                             uint64_t counter, bool want_flags, int64_t& s, bool& f, int64_t& g, int& es, int& ee,
-                                            float (*rec8)[8] = nullptr) {
-  const uint4 x = philox4x32((uint64_t)b, counter, seed);
-  const uint64_t r64 = ((uint64_t)x.x << 32) | x.y;
-  s = (int64_t)__umul64hi(r64, (uint64_t)range);
+                                            float (*rec8)[8] = nullptr, int64_t per_s = 0, uint32_t per_z = 0, uint32_t per_w = 0) {
+  uint4 x;
+  if constexpr (PER) {
+    x = make_uint4(0u, 0u, per_z, per_w);
+    s = per_s;
+  } else {
+    x = philox4x32((uint64_t)b, counter, seed);
+    const uint64_t r64 = ((uint64_t)x.x << 32) | x.y;
+    s = (int64_t)__umul64hi(r64, (uint64_t)range);
+  }
   f = false;
   g = s;
   es = -1;
@@ -925,10 +932,12 @@ __device__ __noinline__ bool scan_row_matches_cold(const GatherArgs& g, int s, i
 }
 
 // TC > 0: the window length is the compile-time constant TC, scalar records are 8 floats and the link records are valid (the launcher
-// checks all three); TC = 0: everything at run time.
-template <bool HASH, bool DRAW, int TC = 0>
+// checks all three); TC = 0: everything at run time.  PER (with DRAW): the start per_s comes from the priority tree (per_descend_chunk),
+// the hindsight streams from per_z / per_w, and the importance weight and the critic weight are written through `pd`.
+template <bool HASH, bool DRAW, int TC = 0, bool PER = false>
 __device__ __forceinline__ void window_scalar_phase(const GatherArgs& g, int64_t b, uint64_t draw_ctr, int& s_out, int& grow_out,
-                                                    int& tail_out) {
+                                                    int& tail_out, const PerDraw* pd = nullptr, int per_s = 0, uint32_t per_z = 0,
+                                                    uint32_t per_w = 0) {
   const ArenaDev& A = g.A;
   const int T = TC > 0 ? TC : g.T;
   const int cap32 = (int)A.capacity, len32 = (int)g.len;
@@ -952,8 +961,12 @@ __device__ __forceinline__ void window_scalar_phase(const GatherArgs& g, int64_t
     bool f;
     int es, ee;
     have0 = HASH && vec8;
-    draw_window<TC>(A, b, device_draw_range(g.counter_dev, g.draw_range, T), g.goal_mode, g.relabel_prob, g.seed, draw_ctr, HASH, s64, f, g64,
-                    es, ee, have0 ? &rv0 : nullptr);
+    if constexpr (PER)  // (counter_dev[2] is not read: the tree holds the eligible range)
+      draw_window<TC, true>(A, b, 0, g.goal_mode, g.relabel_prob, g.seed, draw_ctr, HASH, s64, f, g64, es, ee, have0 ? &rv0 : nullptr, per_s,
+                            per_z, per_w);
+    else
+      draw_window<TC>(A, b, device_draw_range(g.counter_dev, g.draw_range, T), g.goal_mode, g.relabel_prob, g.seed, draw_ctr, HASH, s64, f, g64,
+                      es, ee, have0 ? &rv0 : nullptr);
     if (g.starts_out) g.starts_out[b] = s64;
     if (g.flags_out) g.flags_out[b] = f ? 1 : 0;
     if (g.goal_out) g.goal_out[b] = g64;
@@ -1117,18 +1130,94 @@ __device__ __forceinline__ void window_scalar_phase(const GatherArgs& g, int64_t
       prev_mask = v_mask;
     }
   }
+  // importance weight, only when asked for (beta_dev may be NULL otherwise; critic_weight comes with is_weight); computed after the
+  // window rows so that it is not live across the out-of-line tail scan
+  float isw = 1.f;
+  if constexpr (PER) {
+    if (pd->is_weight != nullptr) {
+      isw = per_is_weight(pd->P.mins[pd->P.n_levels][0], pd->P.leaves[s], pd->beta_dev[0]);
+      pd->is_weight[b] = isw;
+    }
+  }
   if (want_aux && g.aux_weight && T >= 2) {
     // upstream weight of q_loss[t,b]: contig / ((sum_t contig + 1e-4) * B * T)  (deepQlearning.py:222-225,249)
     const float scale = g.inv_bt / (csum + 1e-4f);
     if (T == 2) {
-      st_stream1(g.aux_weight + b, csum * scale);
+      const float wv = csum * scale;
+      st_stream1(g.aux_weight + b, wv);
+      if (PER && pd->critic_weight != nullptr) st_stream1(pd->critic_weight + b, wv * isw);
     } else {
       for (int t = 0; t < T - 1; ++t) {
         float* w = g.aux_weight + (int64_t)t * g.n + b;
-        *w = *w * scale;
+        const float wv = *w * scale;
+        *w = wv;
+        if (PER && pd->critic_weight != nullptr) pd->critic_weight[(int64_t)t * g.n + b] = wv * isw;
       }
     }
   }
+}
+
+// Prioritized draw of the windows cb0 + lane (lane < n_here) of a chunk, for the thread-per-window phase: lane w keeps window w's target
+// and node, and the warp descends through the tree for one window after the other with the descent steps of per_sample_kernel
+// (draw.cuh), so the starts are the same bits.  The root's children are the same for every window and are scanned once per chunk; below
+// it, the children of kPerWindowsInFlight windows are loaded together before their steps.  Returns the start and the last two Philox
+// words of the window (its hindsight streams).
+constexpr int kPerWindowsInFlight = 8;
+__device__ __forceinline__ void per_descend_chunk(const PerDraw& pd, const GatherArgs& g, int64_t cb0, int n_here, uint64_t draw_ctr,
+                                                  int& s_out, uint32_t& z_out, uint32_t& w_out) {
+  constexpr int U = kPerWindowsInFlight;
+  const PerDev& P = pd.P;
+  const int lane = lane_id();
+  const int L = P.n_levels;
+  const int64_t b = cb0 + min(lane, n_here - 1);
+  const uint4 x = philox4x32((uint64_t)b, draw_ctr, g.seed);
+  z_out = x.z;
+  w_out = x.w;
+  double t = per_target(P.sums[L][0], b, g.n, pd.xi != nullptr ? pd.xi[b] : per_uniform(x));
+  int node;
+  {  // root
+    const double v = lane < P.n[L - 1] ? (L == 1 ? (double)P.leaves[lane] : P.sums[L - 1][lane]) : 0.0;
+    double incl, excl;
+    per_scan(v, lane, incl, excl);
+    node = 0;
+    for (int w = 0; w < n_here; ++w) {
+      double tw = shfl_idx_f64(t, w);
+      const int pick = per_pick(v, incl, excl, tw);
+      if (lane == w) {
+        t = tw;
+        node = pick;
+      }
+    }
+  }
+  for (int l = L - 1; l >= 1; --l) {
+    const int64_t n_below = P.n[l - 1];
+    const double* sums = P.sums[l - 1];
+    for (int w0 = 0; w0 < n_here; w0 += U) {
+      int nd[U];
+      double v[U];
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        nd[u] = __shfl_sync(kFull, node, min(w0 + u, n_here - 1));
+        const int64_t c = 32 * (int64_t)nd[u] + lane;
+        v[u] = 0.0;
+        if (c < n_below) v[u] = l == 1 ? (double)__ldg(P.leaves + c) : __ldg(sums + c);
+      }
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int w = w0 + u;
+        if (w >= n_here) break;  // (uniform) the last group of a short chunk
+        double tw = shfl_idx_f64(t, w);
+        double incl, excl;
+        per_scan(v[u], lane, incl, excl);
+        const int pick = per_pick(v[u], incl, excl, tw);
+        if (lane == w) {
+          t = tw;
+          node = 32 * nd[u] + pick;
+        }
+      }
+    }
+  }
+  s_out = node;
 }
 
 // =================================================================================================
@@ -1334,9 +1423,10 @@ __device__ __forceinline__ void lean_store_key(const GatherArgs& g, const int k,
 // among the role's `n_warps` warps of the block (taken through a shuffle by the caller: warp-uniform for the compiler, so the stage
 // bookkeeping and the bulk copies use uniform registers); `blk` / `n_blk`: the block's rank among the blocks that share the windows;
 // `bar_id`: 0 = the role is the whole block, otherwise its named barrier.
-template <bool HASH, bool DRAW, int kLeanStageWindows, int TC = 0, int kStages = 2, int PLAN = 0>
+// `pd` (PER builds): the starts are drawn from this priority tree (per_descend_chunk) instead of uniformly.
+template <bool HASH, bool DRAW, int kLeanStageWindows, int TC = 0, int kStages = 2, int PLAN = 0, bool PER = false>
 __device__ __forceinline__ void gather_lean_body(const GatherArgs& g, unsigned char* lean_smem, const int wib, const int n_warps,
-                                                 const int blk, const int n_blk, const int bar_id) {
+                                                 const int blk, const int n_blk, const int bar_id, const PerDraw* pd = nullptr) {
   const int lane = lane_id();
   const int T = TC > 0 ? TC : g.T;  // (TC: see window_scalar_phase)
   const int len32 = (int)g.len;
@@ -1410,7 +1500,12 @@ __device__ __forceinline__ void gather_lean_body(const GatherArgs& g, unsigned c
 #endif
       if (x == 12345.f) g.aux_mask[0] = x;
     }
-    if (FDQL_DBG(g) & 2) s = (int)(((cb0 + lane) * 7919) % (len32 - T));
+    if constexpr (PER) {
+      int per_s;
+      uint32_t per_z, per_w;
+      per_descend_chunk(*pd, g, cb0, n_here, draw_ctr, per_s, per_z, per_w);
+      if (lane < n_here) window_scalar_phase<HASH, true, TC, true>(g, cb0 + lane, draw_ctr, s, grow, tail_last, pd, per_s, per_z, per_w);
+    } else if (FDQL_DBG(g) & 2) s = (int)(((cb0 + lane) * 7919) % (len32 - T));
     else if (lane < n_here) window_scalar_phase<HASH, DRAW, TC>(g, cb0 + lane, draw_ctr, s, grow, tail_last);
     __syncwarp();
 #pragma unroll 1
@@ -1589,6 +1684,21 @@ fused_pass_kernel(const __grid_constant__ GatherArgs g, const __grid_constant__ 
   }
 }
 
+// The same kernel with prioritized starts (fdql_fused_pass_per): the gather role draws from the priority tree in `pd`; the loss role is
+// the same code.
+template <int FLAGS, bool HASH, int TC = 0, int PLAN = 0>
+__global__ void __launch_bounds__((kFusedLossWarps + kFusedGatherWarps) * 32, 1)
+fused_pass_per_kernel(const __grid_constant__ GatherArgs g, const __grid_constant__ TqcArgs a, const __grid_constant__ PerDraw pd) {
+  extern __shared__ __align__(128) unsigned char fused_smem[];
+  const int w = __shfl_sync(kFull, (int)(threadIdx.x >> 5), 0);
+  constexpr uint32_t kLossBytes = kFusedLossWarps * GrpCfg<128>::kWarpFloatsAlias * sizeof(float);
+  if (w < kFusedLossWarps)
+    tqc_group_body<128, FLAGS>(a, reinterpret_cast<float*>(fused_smem), w, kFusedLossWarps, (int)blockIdx.x, (int)gridDim.x, 1);
+  else
+    gather_lean_body<HASH, true, kFusedStageWindows, TC, kFusedStages, PLAN, true>(g, fused_smem + kLossBytes, w - kFusedLossWarps,
+                                                                                   kFusedGatherWarps, (int)blockIdx.x, (int)gridDim.x, 2, &pd);
+}
+
 int g_tile_override = 0;
 int g_tile_ctas_per_sm = 0;  // tuning hook: resident tile-kernel blocks per SM (0 = as many as fit)
 int g_force_generic_gather = 0;       // tests flip this to cover the descriptor-walking kernel
@@ -1733,15 +1843,27 @@ int launch_gather(const fdql_arena* a, int64_t n, int64_t b_begin, int64_t b_end
     }                                                                                                                       \
     kern<<<(unsigned)a->num_sms, (kFusedLossWarps + kFusedGatherWarps) * 32, smem, st>>>(g, t);                             \
   } while (0)
-#define FDQL_FUSED_FLAGS(HASHV, TCV, PLANV)                          \
+#define FDQL_LAUNCH_FUSED_PER(FLAGSV, HASHV, TCV, PLANV)                                                                    \
+  do {                                                                                                                      \
+    auto kern = fused_pass_per_kernel<FLAGSV, HASHV, TCV, PLANV>;                                                           \
+    static size_t smem_set = 0;                                                                                             \
+    if (smem_set != smem) {                                                                                                 \
+      FDQL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                        \
+      FDQL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)); \
+      smem_set = smem;                                                                                                      \
+    }                                                                                                                       \
+    kern<<<(unsigned)a->num_sms, (kFusedLossWarps + kFusedGatherWarps) * 32, smem, st>>>(g, t, *per);                       \
+  } while (0)
+#define FDQL_FUSED_FLAGS_OF(LAUNCH, HASHV, TCV, PLANV)               \
   do {                                                               \
     switch (flags_) {                                                \
-      case 4: FDQL_LAUNCH_FUSED(4, HASHV, TCV, PLANV); break;        \
-      case 5: FDQL_LAUNCH_FUSED(5, HASHV, TCV, PLANV); break;        \
-      case 6: FDQL_LAUNCH_FUSED(6, HASHV, TCV, PLANV); break;        \
-      default: FDQL_LAUNCH_FUSED(7, HASHV, TCV, PLANV); break;       \
+      case 4: LAUNCH(4, HASHV, TCV, PLANV); break;                   \
+      case 5: LAUNCH(5, HASHV, TCV, PLANV); break;                   \
+      case 6: LAUNCH(6, HASHV, TCV, PLANV); break;                   \
+      default: LAUNCH(7, HASHV, TCV, PLANV); break;                  \
     }                                                                \
   } while (0)
+#define FDQL_FUSED_FLAGS(HASHV, TCV, PLANV) FDQL_FUSED_FLAGS_OF(FDQL_LAUNCH_FUSED, HASHV, TCV, PLANV)
         // TD pairs (T = 2: one transition per window, the shape the learner and the headline use) take the build with the window
         // length, the 8-float scalar record and valid link records known at compile time
         const ArenaDev& D = a->dev;
@@ -1758,11 +1880,19 @@ int launch_gather(const fdql_arena* a, int64_t n, int64_t b_begin, int64_t b_end
         }
         plan |= dg_key << 16;  // (digit 4: the desired_goal key + 1, 0 = none)
         const bool out32 = (uint64_t)T * (uint64_t)n * 16u * FDQL_LEAN_MAXVECS < (1ull << 32);  // (see lean_store_key)
-        if (spec2 && out32 && plan == FDQL_FUSED_PLAN && !(g_force_generic_gather & 4096)) FDQL_FUSED_FLAGS(true, 2, FDQL_FUSED_PLAN);
+        const PerDraw* per = static_cast<const PerDraw*>(draw->per);
+        if (per != nullptr) {  // prioritized: the T = 2 build with the compiled copy plan, else the general build (identical results)
+          if (spec2 && out32 && plan == FDQL_FUSED_PLAN && !(g_force_generic_gather & 4096))
+            FDQL_FUSED_FLAGS_OF(FDQL_LAUNCH_FUSED_PER, true, 2, FDQL_FUSED_PLAN);
+          else if (hash_ok) FDQL_FUSED_FLAGS_OF(FDQL_LAUNCH_FUSED_PER, true, 0, 0);
+          else FDQL_FUSED_FLAGS_OF(FDQL_LAUNCH_FUSED_PER, false, 0, 0);
+        } else if (spec2 && out32 && plan == FDQL_FUSED_PLAN && !(g_force_generic_gather & 4096)) FDQL_FUSED_FLAGS(true, 2, FDQL_FUSED_PLAN);
         else if (spec2) FDQL_FUSED_FLAGS(true, 2, 0);
         else if (hash_ok) FDQL_FUSED_FLAGS(true, 0, 0);
         else FDQL_FUSED_FLAGS(false, 0, 0);
 #undef FDQL_FUSED_FLAGS
+#undef FDQL_FUSED_FLAGS_OF
+#undef FDQL_LAUNCH_FUSED_PER
 #undef FDQL_LAUNCH_FUSED
         FDQL_CUDA(cudaGetLastError());
 #ifdef FDQL_FUSED_ROLE_CLOCK
@@ -1792,6 +1922,7 @@ int launch_gather(const fdql_arena* a, int64_t n, int64_t b_begin, int64_t b_end
       }
     }
   }
+  if (draw != nullptr && draw->per != nullptr) return 1;  // prioritized starts: the fused kernel only, the caller runs the separate launches
   if (lean_ok && (coresident || (g_force_generic_gather & 32))) {
     g.use_link = link_ok64;
     g.log2_gamma = gamma > 0.0 ? log2(gamma) : 0.0;

@@ -333,6 +333,38 @@ int fdql_per_level_view(const fdql_per* per, int32_t level, double** sums, float
 /* every node of the tree from the leaves */
 int fdql_per_rebuild(fdql_per* per, void* stream);
 
+/* fdql_fused_pass with prioritized starts, for the store `per` (T = per->T, the arena is per's): one call does one pass.
+ *   Gather half, batch k+1 (arguments n_windows .. aux_weight, as fdql_fused_pass): the window starts are drawn from the priority tree
+ *   by exactly fdql_per_sample's rules (stratified targets, xi from Philox (b, counter, seed) with the counter_dev protocol or injected,
+ *   the clamp past the last positive leaf, flags / goal rows from the drawn start; counter_dev[2] is not read).  Window b covers rows
+ *   start_b .. start_b + T - 1 (a drawn start is < len - T, so no window wraps; the ring's current length is not baked into the launch, and
+ *   a captured pass keeps gathering the right rows while the ring grows).  It also writes is_weight [n] = (q_min / q[start])^beta with
+ *   beta = beta_dev[0] (is_weight NULL: no weights, and beta_dev is not read and may be NULL) and critic_weight [T-1, n] =
+ *   aux_weight * is_weight (may be NULL; needs FDQL_OPT_EMIT_LEARNER_AUX, aux_weight and is_weight).  aux_weight itself stays the uniform
+ *   reduce weight: the actor and temperature losses take it unweighted.
+ *   Loss half, batch k (arguments M .. stats, as fdql_fused_pass): pass batch k's critic_weight (written by the previous call) as
+ *   grad_scale.  Then, in stream order after the launch that read the tree, the priorities of batch k as fdql_per_update computes them,
+ *   from loss_starts (batch k's starts, written by the previous call), this call's per-transition loss and loss_contig (batch k's
+ *   is_contiguous, may be NULL): M / (T - 1) windows.
+ * M == 0: the gather alone, no update; n_windows == 0: the loss and the update alone.  Rows recorded by writers are applied first, on
+ * `stream`, never under capture (as every PER call).
+ * Staleness: the draw of batch j sees the priorities of batches <= j - 2 (batch j - 1's loss runs in the same call as batch j's draw):
+ * the one-batch lag that any overlap of sampling with the loss implies.  Callers that need the priorities of batch j - 1 in draw j call
+ * fdql_per_update before fdql_per_sample instead.
+ * Double buffers: call k writes the gather outputs, starts, is_weight and critic_weight of batch k+1 while its loss reads those of batch
+ * k, so each of them needs two sets, swapped every call.  Shapes the fused kernel does not serve run as fdql_per_sample, the co-resident
+ * fdql_sample_gather on its streams, critic_weight, fdql_tqc_loss and the update, with identical results.
+ * FDQL_EINVAL: NULL per, a loss half without loss_starts or loss, critic_weight without FDQL_OPT_EMIT_LEARNER_AUX; FDQL_EOVERSAMPLE as
+ * fdql_per_sample. */
+int fdql_fused_pass_per(fdql_per* per, int64_t n_windows, int32_t goal_mode, float relabel_prob, uint64_t seed, uint64_t counter,
+                        uint64_t* counter_dev, const double* xi, const float* beta_dev, int64_t* starts, uint8_t* flags, int64_t* goal_rows,
+                        float* is_weight, float* critic_weight, int32_t reward_op, const float* reward_params_host, int32_t n_params,
+                        double gamma, uint32_t opts, int32_t batch_for_weight, float* const* out, float* aux_mask, float* aux_contig,
+                        float* aux_weight, int64_t M, int32_t n_atoms, int32_t n_drop, const float* next_z, const float* q_pred,
+                        const float* next_log_pi, const float* reward, const float* mask, const float* mc_return, const float* grad_scale,
+                        float alpha, float loss_gamma, float* loss, float* grad_q, double* stats, const int64_t* loss_starts,
+                        const float* loss_contig, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

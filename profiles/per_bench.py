@@ -5,11 +5,15 @@
                                   windows), CUDA events over 20 replays of a graph holding 50 launches (launch gaps excluded);
   updates_per_s                   whole learner steps (bench.py's second metric, the step captured in one CUDA graph) with PER off and
                                   on, in the same process, alternated;
-  pass_transitions_per_s          64 x 4096 windows: the uniform fused pass (fdql_fused_pass, bench.py's headline) beside a PER pass
-                                  (fdql_per_sample + injected fdql_sample_gather + fdql_tqc_loss + fdql_per_update), graphed.
+  pass                            64 x 4096 windows: the uniform fused pass (fdql_fused_pass, bench.py's headline) beside a PER pass
+                                  as four launches (fdql_per_sample + injected fdql_sample_gather + fdql_tqc_loss + fdql_per_update),
+                                  graphed, and the four launches timed one by one (`split_ms`);
+  fused_per                       the same 64 x 4096 windows through fdql_fused_pass_per (prioritized draw in the gather role, update
+                                  after the launch) against the uniform fused pass, alternated in one run: median and spread over repeats.
 
-The card name and its power limit are read in the same run: the numbers belong to that card at that limit.
-    python profiles/per_bench.py [--ring-rows 10000000]"""
+The card name, its power limit and the SM clock are read in the same run: the numbers belong to that card at that limit.
+    python profiles/per_bench.py [--ring-rows 10000000] [--split-only]   (--split-only: the four-launch split alone, which every
+                                                                          build with fdql_per_* can run)"""
 import argparse
 import ctypes as C
 import json
@@ -27,9 +31,9 @@ def card():
     import torch
     out = {"name": torch.cuda.get_device_name(0)}
     try:
-        q = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader,nounits", "-i", "0"],
+        q = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm,clocks.sm", "--format=csv,noheader,nounits", "-i", "0"],
                            capture_output=True, text=True, timeout=30).stdout.strip().split(",")
-        out["power_limit_w"], out["sm_max_mhz"] = float(q[0]), float(q[1])
+        out["power_limit_w"], out["sm_max_mhz"], out["sm_mhz_now"] = float(q[0]), float(q[1]), float(q[2])
     except Exception as e:  # the numbers stand without it, but say so
         out["power_limit_w"] = f"unavailable: {e}"
     return out
@@ -64,6 +68,8 @@ def main():
     ap.add_argument("--ring-rows", type=int, default=10_000_000)
     ap.add_argument("--passes", type=int, default=64, help="batches of 4096 windows per pass")
     ap.add_argument("--updates", type=int, default=60)
+    ap.add_argument("--split-only", action="store_true", help="only the per-launch split of the four-launch PER pass")
+    ap.add_argument("--repeats", type=int, default=7, help="alternations of the uniform and the prioritized fused pass")
     args = ap.parse_args()
     import torch
     import fastdeepqlearning_b200 as pkg
@@ -95,8 +101,17 @@ def main():
 
     def update():
         L.check(lib.fdql_per_update(ring._per, B, p(st), p(loss), None, C.c_void_p(torch.cuda.current_stream().cuda_stream)))
-    res["per_sample_ms"] = graph_ms(torch, sample)
-    res["per_update_ms"] = graph_ms(torch, update)
+    if not args.split_only:
+        res["per_sample_ms"] = graph_ms(torch, sample)
+        res["per_update_ms"] = graph_ms(torch, update)
+        learner_rates(torch, Agent, SampleTimeHindsight, ring, args, res)
+    pass_rates(torch, lib, L, ring, args, res, p)
+    res["card_after"] = card()
+    print(json.dumps(res))
+
+
+def learner_rates(torch, Agent, SampleTimeHindsight, ring, args, res):
+    B, T, CQ = bench.B, bench.T, bench.CQ
 
     # ---- learner updates/s, PER off and on, alternated
     def learner(per):
@@ -127,6 +142,10 @@ def main():
                       "spread_ms": {"uniform": [min(ms[False]), max(ms[False])], "per": [min(ms[True]), max(ms[True])]}}
     del learners
 
+
+def pass_rates(torch, lib, L, ring, args, res, p):
+    B, T, CQ = bench.B, bench.T, bench.CQ
+    dev = torch.device("cuda:0")
     # ---- a pass of 64 x 4096 windows: uniform fused pass vs PER pass
     n = args.passes * B
     M = (T - 1) * n
@@ -168,11 +187,52 @@ def main():
         L.check(lib.fdql_per_update(ring._per, n, p(sts), p(ploss), p(contig), sp()))
     t_per = graph_ms(torch, per_pass, per_graph=10, reps=10)  # (also leaves a gathered batch in the first set for the fused loss)
     t_fused = graph_ms(torch, fused, per_graph=10, reps=10)
+    # the four launches of the PER pass one by one (each graphed alone; the inputs are those the pass above left)
+
+    def l_sample():
+        L.check(lib.fdql_per_sample(ring._per, n, L.GOAL_FUTURE, bench.P_RELABEL, 7, 0, p(ctr), None, p(ring._per_beta), p(sts), p(fls), p(gos),
+                                    p(isw), sp()))
+
+    def l_gather():
+        L.check(lib.fdql_sample_gather(ring._h, n, T, ring._maxlen, p(sts), p(fls), p(gos), ring.reward_op.op, params, n_params, bench.GAMMA,
+                                       opts, B, outp, p(mask), p(contig), p(weight), sp()))
+
+    def l_loss():
+        L.check(lib.fdql_tqc_loss(M, CQ, bench.N_DROP, p(z), p(q), p(lp), p(out["reward"][1:]), p(mask[1:]), p(out["mc_return"][1:]),
+                                  p(weight), bench.ALPHA, bench.GAMMA, p(ploss), p(grad), None, p(stats), sp()))
+
+    def l_update():
+        L.check(lib.fdql_per_update(ring._per, n, p(sts), p(ploss), p(contig), sp()))
+    split = {name: graph_ms(torch, fn, per_graph=10, reps=10) for name, fn in
+             (("per_sample", l_sample), ("sample_gather", l_gather), ("tqc_loss", l_loss), ("per_update", l_update))}
     res["pass"] = {"windows": n, "uniform_fused_ms": t_fused, "per_ms": t_per, "uniform_fused_transitions_per_s": M / t_fused * 1e3,
-                   "per_transitions_per_s": M / t_per * 1e3,
+                   "per_transitions_per_s": M / t_per * 1e3, "split_ms": split,
                    "note": "the uniform pass fuses loss k with gather k+1 in one launch; the PER pass is four launches in stream order, "
                            "the gather as the injected-stream kernel"}
-    print(json.dumps(res))
+    if args.split_only or not hasattr(lib, "fdql_fused_pass_per"):
+        return
+
+    # ---- fdql_fused_pass_per: loss + update of one batch, prioritized gather of the next, against the uniform fused pass, alternated.
+    # Call k reads batch k's set (critic weight as grad_scale, starts and is_contiguous for the update) and writes batch k+1's set.
+    isw2, crit, crit2 = torch.empty_like(isw), torch.empty_like(weight), torch.empty_like(weight)
+    sts2 = torch.empty_like(sts)
+    crit.copy_(weight)
+
+    def fused_per():
+        L.check(lib.fdql_fused_pass_per(ring._per, n, L.GOAL_FUTURE, bench.P_RELABEL, 7, 0, p(ctr), None, p(ring._per_beta), p(sts2), p(fls),
+                                        p(gos), p(isw2), p(crit2), ring.reward_op.op, params, n_params, bench.GAMMA, opts, B, outp2, p(mask2),
+                                        p(contig2), p(weight2), M, CQ, bench.N_DROP, p(z), p(q), p(lp), p(out["reward"][1:]), p(mask[1:]),
+                                        p(out["mc_return"][1:]), p(crit), bench.ALPHA, bench.GAMMA, p(ploss), p(grad), p(stats), p(sts),
+                                        p(contig), sp()))
+    ms = {"uniform": [], "per": []}
+    for _ in range(args.repeats):
+        ms["uniform"].append(graph_ms(torch, fused, per_graph=10, reps=10))
+        ms["per"].append(graph_ms(torch, fused_per, per_graph=10, reps=10))
+    med = {k: sorted(v)[len(v) // 2] for k, v in ms.items()}
+    res["fused_per"] = {"windows": n, "uniform_fused_ms": med["uniform"], "per_fused_ms": med["per"], "ratio": med["per"] / med["uniform"],
+                        "per_fused_transitions_per_s": M / med["per"] * 1e3,
+                        "spread_ms": {k: [min(v), max(v)] for k, v in ms.items()}, "repeats": args.repeats,
+                        "note": "per_fused_ms = the fused launch (loss k + prioritized gather k+1) plus the priority update of batch k"}
 
 
 if __name__ == "__main__":
