@@ -4,7 +4,11 @@ state equals the goal; reward -1 until then): vectorised numpy bit-flip envs -> 
 commit, link records) -> `Learner.train_step` (sample-time "future" hindsight relabelling, fused TQC loss, discrete Gumbel-softmax
 actor with the one-hot kernel, whole step as a CUDA graph).  Prints the greedy success rate as it trains.
 
-    python examples/train_bitflip_her.py --bits 10 --updates 4000 [--per]
+With --torch-reward the reward is the bit-flip function written in PyTorch (a TorchReward) instead of the device functor, and
+hindsight relabelling moves to write time (her_mode "random": one relabelled copy of every episode, made when it is flushed),
+because sample-time relabelling evaluates the reward inside the gather kernels.
+
+    python examples/train_bitflip_her.py --bits 10 --updates 4000 [--per] [--torch-reward]
 """
 import argparse
 import os
@@ -53,6 +57,12 @@ def rollout(actor, n_envs, bits, horizon, device, greedy, rng, eps=0.0):
     return rows, success
 
 
+def bitflip_reward(achieved_goal, goal):
+    """franQ/Env/bitflip.py:143-152 in PyTorch, batched over rows: reward 0 when every bit matches, else -1; done on a match."""
+    hit = (achieved_goal == goal).all(-1)
+    return hit.float() - 1.0, hit
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--bits", type=int, default=10)
@@ -61,6 +71,7 @@ def main():
     ap.add_argument("--batch", type=int, default=1024)
     ap.add_argument("--eps", type=float, default=0.2)
     ap.add_argument("--per", action="store_true", help="prioritized replay (use_prioritized_replay=True)")
+    ap.add_argument("--torch-reward", action="store_true", help="reward as a TorchReward, write-time hindsight (her_mode='random')")
     args = ap.parse_args()
     device = torch.device("cuda:0")
     rng = np.random.default_rng(0)
@@ -69,9 +80,10 @@ def main():
     conf = Agent.LearnerConf(training_device="cuda:0", obs_space={"obs_1d": bits, "achieved_goal": bits, "desired_goal": bits},
                              action_space=types.SimpleNamespace(n=bits, shape=()), discrete=True, num_critics=5, num_q_predictions=10,
                              top_quantiles_to_drop=0.2, batch_size=args.batch, temporal_len=2, replay_size=200_000, use_HER=True,
-                             her_mode="future", num_instances=1, gamma=0.98, learning_rate=1e-3, use_cuda_graph=True,
+                             her_mode="random" if args.torch_reward else "future", num_instances=1, gamma=0.98, learning_rate=1e-3, use_cuda_graph=True,
                              use_prioritized_replay=args.per, per_beta_steps=args.updates)
-    read, write = Replay.make(conf, compute_reward=fdql.RewardOp.bitflip())
+    reward = fdql.TorchReward(bitflip_reward) if args.torch_reward else fdql.RewardOp.bitflip()
+    read, write = Replay.make(conf, compute_reward=reward)
     learner = Agent.Learner(conf, read)
     actor = learner.actor_critic.actor
     t0, updates = time.time(), 0

@@ -3,11 +3,13 @@
 from .async_replay_memory import AsyncReplayMemory
 from .replay_memory import ReplayMemory, OversampleError
 from . import wrappers
+from ..reward_ops import RewardOp, require_device_functor
 
 
 def make(conf, **kwargs):
     """Replay/__init__.py:8-38.  Composition order is the reference's: NStepReturn (inner) -> SquashRewards -> HER (outer).
-    `kwargs["compute_reward"]` must be a device reward functor (fastdeepqlearning_b200.RewardOp)."""
+    `kwargs["compute_reward"]` is a device reward functor (fastdeepqlearning_b200.RewardOp) or, for the write-time modes
+    ("final", "random", "vmap"), a fastdeepqlearning_b200.TorchReward."""
     device = getattr(conf, "training_device", "cuda:0")
     shards = [AsyncReplayMemory(int(conf.replay_size), conf.batch_size, conf.temporal_len, device=device)
               for _ in range(conf.num_instances)]
@@ -32,6 +34,7 @@ def make(conf, **kwargs):
             write_heads = [wrappers.HindsightVmapWrite(r, kwargs["compute_reward"]) for r in write_heads]
             read_heads = [wrappers.HindsightVmapRead(r) for r in read_heads]
         elif her_mode == "future":  # sample-time relabelling (BASELINE.json configs[2]); rows are stored once
+            require_device_functor(RewardOp.coerce(kwargs["compute_reward"]), "her_mode='future' (sample-time relabelling)")
             for r in shards:
                 r.replay.set_reward_op(kwargs["compute_reward"], conf.gamma)
             read_heads = [wrappers.SampleTimeHindsight(r, relabel_prob=getattr(conf, "her_relabel_prob", 0.8)) for r in read_heads]

@@ -21,7 +21,7 @@ import torch
 
 from .. import _lib as L
 from .._lib import OversampleError, check
-from ..reward_ops import RewardOp
+from ..reward_ops import RewardOp, TorchReward, require_device_functor
 
 
 def _locked(fn):
@@ -72,7 +72,7 @@ class ReplayMemory:
         self.squash_rewards = False  # Pohlen transform of the reward column inside the append kernel (wrappers.SquashRewards)
         self._pending_eps: T.List[T.Tuple[int, int]] = []  # (first row, length) of finished, uncommitted episodes
         self._open_ep_first, self._open_ep_len = 0, 0
-        self.reward_op: T.Optional[RewardOp] = None
+        self.reward_op: T.Union[RewardOp, TorchReward, None] = None
         self.gamma = 0.99
         self._rng_seed = int(kwargs.get("seed", 0x5EED))
         self._rng_counter = 0
@@ -117,6 +117,7 @@ class ReplayMemory:
         self.squash_rewards = bool(on)
 
     def set_reward_op(self, op, gamma=None):
+        """The reward of hindsight relabelling: a RewardOp (every mode) or a TorchReward (write-time flushes only)."""
         self.reward_op = RewardOp.coerce(op)
         if gamma is not None:
             self.gamma = float(gamma)
@@ -202,8 +203,9 @@ class ReplayMemory:
 
     @_locked
     def commit_episodes(self, begins: torch.Tensor, lens: torch.Tensor, with_returns=False, gamma=None):
-        """Record episode extents (and optionally return-to-go, nstep_return.py:60-72) for episodes already in the ring."""
-        op = self.reward_op or RewardOp(L.REWARD_NONE)
+        """Record episode extents (and optionally return-to-go, nstep_return.py:60-72) for episodes already in the ring.  With a
+        TorchReward the scan records carry no goal-agnostic reward: those serve sample-time relabelling, which needs a RewardOp."""
+        op = self.reward_op if isinstance(self.reward_op, RewardOp) else RewardOp(L.REWARD_NONE)
         params, n_params = op.c_params()
         check(self._lib.fdql_commit_episodes(self._h, int(begins.numel()), C.c_void_p(begins.data_ptr()),
                                              C.c_void_p(lens.data_ptr()), float(self.gamma if gamma is None else gamma),
@@ -256,17 +258,50 @@ class ReplayMemory:
         first = C.c_int64()
         check(self._lib.fdql_arena_reserve(self._h, total, C.byref(first)))
         self._advance(total)
-        params, n_params = self.reward_op.c_params()
         src = torch.as_tensor(src_begins, dtype=torch.int64).to(self.device)
         goal = torch.as_tensor(goal_rows, dtype=torch.int64).to(self.device)
         dst_d = dst.to(self.device)
         lens_d = lens_t.to(device=self.device, dtype=torch.int32)
+        gam = float(self.gamma if gamma is None else gamma)
+        if isinstance(self.reward_op, TorchReward):
+            # R(ag_j, g*) and R(ag_j, dg_j) of every source row, packed episode after episode, from ONE call of the user's function
+            rows = self._episode_rows(src_begins, lens_t)
+            n = rows.numel()
+            ag, dg = self._gather_goals(torch.cat([rows, goal]))
+            gstar = ag[n:].repeat_interleave(lens_t.to(self.device), dim=0, output_size=n)
+            r, d = self.reward_op(torch.cat([ag[:n], ag[:n]]), torch.cat([gstar, dg[:n]]))
+            check(self._lib.fdql_her_flush_episodes_given(self._h, int(lens_t.numel()), C.c_void_p(src.data_ptr()),
+                                                          C.c_void_p(lens_d.data_ptr()), C.c_void_p(dst_d.data_ptr()),
+                                                          C.c_void_p(goal.data_ptr()), n, C.c_void_p(r.data_ptr()),
+                                                          C.c_void_p(d.data_ptr()), C.c_void_p(r[n:].data_ptr()), gam,
+                                                          int(bool(with_returns)), _stream_ptr(self.device)))
+            return dst
+        params, n_params = self.reward_op.c_params()
         check(self._lib.fdql_her_flush_episodes(self._h, int(lens_t.numel()), C.c_void_p(src.data_ptr()),
                                                 C.c_void_p(lens_d.data_ptr()), C.c_void_p(dst_d.data_ptr()),
-                                                C.c_void_p(goal.data_ptr()), self.reward_op.op, params, n_params,
-                                                float(self.gamma if gamma is None else gamma), int(bool(with_returns)),
-                                                _stream_ptr(self.device)))
+                                                C.c_void_p(goal.data_ptr()), self.reward_op.op, params, n_params, gam,
+                                                int(bool(with_returns)), _stream_ptr(self.device)))
         return dst
+
+    def _episode_rows(self, begins, lens):
+        """Ring rows of whole episodes, episode after episode, each oldest row first (the packed order of the *_given entry points)."""
+        lens = np.asarray(lens, dtype=np.int64)
+        first = np.repeat(np.asarray(begins, dtype=np.int64) - np.cumsum(lens) + lens, lens)
+        return torch.from_numpy((first + np.arange(int(lens.sum()))) % self._maxlen).to(self.device)
+
+    def _gather_goals(self, rows):
+        """(achieved_goal, desired_goal) [n, G] of ring rows `rows` (device int64 [n]), gathered by fdql_gather_rows."""
+        n = rows.numel()
+        roles = [self._role_override.get(k, L.ROLE_BY_NAME.get(k, L.ROLE_NONE)) for k in self._keys]
+        if L.ROLE_ACHIEVED_GOAL not in roles or L.ROLE_DESIRED_GOAL not in roles:
+            raise ValueError("hindsight relabelling needs achieved_goal and desired_goal keys")
+        ka, kd = roles.index(L.ROLE_ACHIEVED_GOAL), roles.index(L.ROLE_DESIRED_GOAL)
+        ag = torch.empty((n, self._widths[ka]), dtype=torch.float32, device=self.device)
+        dg = torch.empty((n, self._widths[kd]), dtype=torch.float32, device=self.device)
+        out = [0] * len(self._keys)
+        out[ka], out[kd] = ag.data_ptr(), dg.data_ptr()
+        check(self._lib.fdql_gather_rows(self._h, n, C.c_void_p(rows.data_ptr()), L.ptr_array(out), _stream_ptr(self.device)))
+        return ag, dg
 
     # ------------------------------------------------------------------ "vmap" hindsight variant (her_vmap.py, nstep_return_vmap.py)
     VMAP_KEYS = ("virtual_goals", "virtual_rewards", "virtual_dones", "virtual_mc_return")
@@ -294,12 +329,28 @@ class ReplayMemory:
             V = self._widths[kr] - 1
             if picks.numel() != b.numel() * V:
                 raise ValueError(f"pick_rows must hold {V} rows per episode")
-        op = self.reward_op or RewardOp(L.REWARD_NONE)
+        gam = float(self.gamma if gamma is None else gamma)
+        mode = (1 if fill else 0) | (2 if returns else 0)
+        if fill and isinstance(self.reward_op, TorchReward):
+            # the [n_rows, V+1] grid: R(ag, virtual goal v) in columns v < V, R(ag, dg) in column V, from ONE call of the user's function
+            lens_np = np.asarray(lens, dtype=np.int64)
+            rows = self._episode_rows(begins, lens_np)
+            n = rows.numel()
+            ag, dg = self._gather_goals(torch.cat([rows, picks.reshape(-1)]))
+            G = ag.shape[1]
+            vg = ag[n:].reshape(b.numel(), V, G).repeat_interleave(l.long(), dim=0, output_size=n)
+            goals = torch.cat([vg, dg[:n, None]], dim=1).reshape(n * (V + 1), G)
+            r, d = self.reward_op(ag[:n, None].expand(n, V + 1, G).reshape(n * (V + 1), G), goals)
+            check(self._lib.fdql_vmap_flush_episodes_given(self._h, int(b.numel()), C.c_void_p(b.data_ptr()), C.c_void_p(l.data_ptr()),
+                                                           C.c_void_p(picks.data_ptr()), kg, kr, kd, kret if returns else -1, n,
+                                                           C.c_void_p(r.data_ptr()), C.c_void_p(d.data_ptr()), gam, mode,
+                                                           int(bool(done_quirk)), _stream_ptr(self.device)))
+            return
+        op = self.reward_op if isinstance(self.reward_op, RewardOp) else RewardOp(L.REWARD_NONE)
         params, n_params = op.c_params()
         check(self._lib.fdql_vmap_flush_episodes(self._h, int(b.numel()), C.c_void_p(b.data_ptr()), C.c_void_p(l.data_ptr()),
                                                  C.c_void_p(picks.data_ptr()) if picks is not None else None, kg, kr, kd,
-                                                 kret if returns else -1, op.op, params, n_params,
-                                                 float(self.gamma if gamma is None else gamma), (1 if fill else 0) | (2 if returns else 0),
+                                                 kret if returns else -1, op.op, params, n_params, gam, mode,
                                                  int(bool(done_quirk)), _stream_ptr(self.device)))
 
     @_locked
@@ -476,10 +527,18 @@ class ReplayMemory:
         check(self._lib.fdql_arena_link_state(self._h, 0, C.byref(gam), C.byref(st)))
         return {"maxlen": self._maxlen, "keys": list(self._keys), "widths": list(self._widths), "shapes": dict(self._shapes),
                 "top": self._top, "len": self._curr_len, "gamma": self.gamma, "link": (gam.value, st.value),
-                "reward_op": None if self.reward_op is None else (self.reward_op.op, list(self.reward_op.params or [])),
+                "reward_op": self._reward_op_state(),
                 "memory": {k: v.cpu().clone() for k, v in self.memory.items()}, "ep_start": es.cpu().clone(), "ep_end": ee.cpu().clone(),
                 "scan": self._meta_rows(2).view(torch.int32).cpu().clone(), "links": self._meta_rows(3).view(torch.int32).cpu().clone(),
                 "per": self._per_state()}
+
+    def _reward_op_state(self):
+        """(op, params) of a RewardOp; "torch" for a TorchReward, whose function is not pickled (set it again before restoring)."""
+        if self.reward_op is None:
+            return None
+        if isinstance(self.reward_op, TorchReward):
+            return "torch"
+        return (self.reward_op.op, list(self.reward_op.params or []))
 
     def _per_state(self):
         if self._per is None:
@@ -494,9 +553,12 @@ class ReplayMemory:
             raise RuntimeError("load_state_dict needs a fresh ReplayMemory")
         if int(sd["maxlen"]) != self._maxlen:
             raise ValueError(f"snapshot of a ring of {sd['maxlen']} rows, this one has {self._maxlen}")
+        if sd["reward_op"] == "torch" and not isinstance(self.reward_op, TorchReward):
+            raise ValueError("the snapshot's reward is a TorchReward, whose function a snapshot does not carry: call "
+                             "set_reward_op(TorchReward(fn)) (or build the ring through its hindsight wrapper) before load_state_dict")
         self._jit_initialize(dict(zip(sd["keys"], sd["widths"])), sd["shapes"])
         self.gamma = float(sd["gamma"])
-        if sd["reward_op"] is not None:
+        if sd["reward_op"] is not None and sd["reward_op"] != "torch":
             self.reward_op = RewardOp(sd["reward_op"][0], sd["reward_op"][1] or ())
         dev = [sd["memory"][k].to(self.device, dtype=torch.float32).reshape(self._maxlen, w).contiguous()
                for k, w in zip(self._keys, self._widths)]
@@ -641,6 +703,8 @@ class ReplayMemory:
         also carries `mask`, `is_contiguous` and `loss_weight` (deepQlearning.py:201-203,222-225).
         `prioritized=True` (after enable_priorities) draws the starts by priority (draw_prioritized: `beta`, `xi`) and gathers them
         with the same kernel as injected starts; the dict then also carries `is_weight` [B] and the `starts` [B] drawn."""
+        if relabel_prob > 0:
+            require_device_functor(self.reward_op, "sample-time relabelling (relabel_prob > 0)")
         if prioritized:
             if starts is not None or length is not None:
                 raise ValueError("prioritized sampling draws its own starts")
@@ -678,6 +742,7 @@ class ReplayMemory:
             goal_rows = self._to_dev_i64(goal_rows)
             if self.reward_op is None:
                 raise ValueError("relabelling needs set_reward_op(...)")
+            require_device_functor(self.reward_op, "sample-time relabelling")
         out = self._outputs((Tn, n), reuse=reuse_outputs, exclude=tuple(exclude_keys))
         opts = (L.OPT_EXACT_EPISODE_STEP if exact_episode_step else 0) | (L.OPT_EMIT_LEARNER_AUX if aux else 0)
         aux_t = [None, None, None]
@@ -691,7 +756,7 @@ class ReplayMemory:
                          torch.empty((Tn - 1, n, 1), dtype=torch.float32, device=self.device)]
                 if reuse_outputs:
                     self._out_cache[ck] = aux_t
-        op = self.reward_op or RewardOp(L.REWARD_NONE)
+        op = self.reward_op if isinstance(self.reward_op, RewardOp) else RewardOp(L.REWARD_NONE)
         params, n_params = op.c_params()
         if fused:
             check(self._lib.fdql_sample_gather_draw(

@@ -4,12 +4,13 @@ form used by the B200 path (mode "future", relabel probability k/(k+1)).
 Write-time: the episode in flight is held on the host; at `episode_done` the real rows go to the ring in one batch and
 the hindsight copy (goal substitution, reward recompute, synthetic-episode splitting of task_done / episode_step, and
 the inner NStepReturn's return over the relabelled rewards) is produced on the device by fdql_her_flush_episodes.
-`compute_reward` is a device functor (RewardOp); the goal pick uses Python's `random` like her.py:51-53."""
+`compute_reward` is a device functor (RewardOp) or a TorchReward; with the latter the ring evaluates it once per flush on the
+gathered goals and fdql_her_flush_episodes_given consumes the results.  The goal pick uses Python's `random` like her.py:51-53."""
 import random
 
 from .wrapper_base_class import ReplayMemoryWrapper
 from .nstep_return import stack_rows
-from ...reward_ops import RewardOp
+from ...reward_ops import RewardOp, require_device_functor
 
 
 class HindsightNStepReplay(ReplayMemoryWrapper):
@@ -65,6 +66,7 @@ class SampleTimeHindsight(ReplayMemoryWrapper):
 
     def __init__(self, replay_buffer, relabel_prob=0.8, goal_mode=None, aux=True):
         ReplayMemoryWrapper.__init__(self, replay_buffer)
+        require_device_functor(getattr(replay_buffer, "reward_op", None), "SampleTimeHindsight")
         self.relabel_prob, self.goal_mode, self.aux = relabel_prob, goal_mode, aux
 
     def temporal_sample(self, *args, **kwargs):

@@ -5,7 +5,8 @@ for the whole batch.
 Write head: the episode in flight is held on the host; at `episode_done` its rows go to the ring in one batch and the
 virtual columns are produced on the device by fdql_vmap_flush_episodes (the reference runs a jax.vmap over goals on the host
 and then pushes rows one by one through Python).  The goal picks use `np.random.randint(0, L, V)` like her_vmap.py:75.
-Read head: fdql_vmap_select_column reads only the chosen column.  `compute_reward` is a device functor (RewardOp)."""
+Read head: fdql_vmap_select_column reads only the chosen column.  `compute_reward` is a device functor (RewardOp) or a TorchReward,
+which the ring evaluates once per flush over the [L, V+1] grid of (row, goal) pairs for fdql_vmap_flush_episodes_given."""
 import random
 
 import numpy as np

@@ -4,9 +4,9 @@ Host-side mirror of the reference's `franQ.Replay` and `franQ.Agent.components` 
 (hand-written CUDA behind the C ABI in include/fdql.h).  No CPU fallback: importing is cheap, but every
 operation needs the built library and a CUDA device and fails loudly otherwise."""
 from ._lib import lib, FdqlError, OversampleError, LIB_PATH, EXPORTS  # noqa: F401
-from .reward_ops import RewardOp  # noqa: F401
+from .reward_ops import RewardOp, TorchReward  # noqa: F401
 
-__all__ = ["lib", "FdqlError", "OversampleError", "RewardOp", "Replay", "Agent", "Runner"]
+__all__ = ["lib", "FdqlError", "OversampleError", "RewardOp", "TorchReward", "Replay", "Agent", "Runner"]
 
 
 def __getattr__(name):  # lazy: the sub-packages import torch

@@ -59,6 +59,8 @@ _SIGNATURES = {
     "fdql_vmap_flush_episodes": (C.c_int, [_p, _i32, _p, _p, _p, _i32, _i32, _i32, _i32, _i32, C.POINTER(_f32), _i32, _f64, _i32, _i32, _p]),
     "fdql_vmap_select_column": (C.c_int, [_p, _i64, _i32, _i64, _p, _i32, _i32, _i32, _i32, _i32, _i32, _p, _p, _p, _p, _p, _p, _p, _p]),
     "fdql_q3_duplicate": (C.c_int, [_p, _i64, _i32, _i64, _f64, _p]),
+    "fdql_her_flush_episodes_given": (C.c_int, [_p, _i32, _p, _p, _p, _p, _i64, _p, _p, _p, _f64, _i32, _p]),
+    "fdql_vmap_flush_episodes_given": (C.c_int, [_p, _i32, _p, _p, _p, _i32, _i32, _i32, _i32, _i64, _p, _p, _f64, _i32, _i32, _p]),
     "fdql_arena_reserve": (C.c_int, [_p, _i64, C.POINTER(_i64)]),
     "fdql_sample_streams": (C.c_int, [_p, _i64, _i32, _i32, _f32, _u64, _u64, _p, _p, _p, _p, _p]),
     "fdql_gather_rows": (C.c_int, [_p, _i64, _p, _pp, _p]),

@@ -4,6 +4,8 @@
 #include <stdarg.h>
 #include <stdlib.h>
 
+#include <vector>
+
 #include "common.cuh"
 #include "goal_eval.cuh"
 
@@ -213,20 +215,25 @@ commit_kernel(ArenaDev A, int32_t n_eps, const int64_t* __restrict__ ep_begin, c
 }
 
 // -------------------------------------------------------------------------------------------------
-// write-time hindsight copy, her.py:55-95 (+ the inner NStepReturn flush, quirk Q5): one warp per episode
+// write-time hindsight copy, her.py:55-95 (+ the inner NStepReturn flush, quirk Q5): one warp per episode.
+// Reward = RewardSpec evaluates R(ag_j, g*) and R(ag_j, dg_j) with the device functor; GivenReward loads them (common.cuh).
 // -------------------------------------------------------------------------------------------------
-template <int LPR>
+template <int LPR, class Reward>
 __global__ void __launch_bounds__(256)
 her_flush_kernel(ArenaDev A, int32_t n_eps, const int64_t* __restrict__ src_begin, const int32_t* __restrict__ ep_len,
-                 const int64_t* __restrict__ dst_begin, const int64_t* __restrict__ goal_row, RewardSpec rs, double gamma,
+                 const int64_t* __restrict__ dst_begin, const int64_t* __restrict__ goal_row, Reward rw, double gamma,
                  int with_returns) {
+  constexpr bool given = kGivenReward<Reward>;
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = lane_id();
   if (warp >= n_eps) return;
   const int64_t s = src_begin[warp], d0 = dst_begin[warp], grow = goal_row[warp];
   const int L = ep_len[warp];
   const int64_t dend = ring_row(d0, L - 1, A.capacity);
-  const float4 gstar = load_goal_slice<LPR>(A, grow);
+  float4 gstar;
+  int64_t p0 = 0;  // first packed row of this episode (GivenReward)
+  if constexpr (given) p0 = packed_first_row(ep_len, warp);
+  else gstar = load_goal_slice<LPR>(A, grow);
   // wide keys: verbatim copy, except desired_goal := g*
   for (int w = 0; w < A.n_wide; ++w) {
     const WideSlab W = A.wide[w];
@@ -245,10 +252,17 @@ her_flush_kernel(ArenaDev A, int32_t n_eps, const int64_t* __restrict__ src_begi
     const int j = jb + lane;
     const bool valid = j < L;
     float Rg, Rdg = 0.f;
-    bool dn, dtmp, has_nan;
+    bool dn, has_nan;
     uint64_t h;
-    eval_chunk<LPR, false>(A, rs, s, jb, L - 1, gstar, Rg, dn);
-    if (A.wide_dg >= 0) eval_chunk<LPR, true>(A, rs, s, jb, L - 1, gstar, Rdg, dtmp);
+    if constexpr (given) {
+      Rg = valid ? rw.reward[p0 + j] : 0.f;
+      dn = valid && rw.done[p0 + j] != 0;
+      Rdg = valid ? rw.reward_dg[p0 + j] : 0.f;
+    } else {
+      bool dtmp;
+      eval_chunk<LPR, false>(A, rw, s, jb, L - 1, gstar, Rg, dn);
+      if (A.wide_dg >= 0) eval_chunk<LPR, true>(A, rw, s, jb, L - 1, gstar, Rdg, dtmp);
+    }
     hash_chunk<LPR>(A, s, jb, L - 1, h, has_nan);  // achieved_goal is copied verbatim: same hash as the source row
     const unsigned bal = __ballot_sync(kFull, valid && dn);
     if (valid) {
@@ -369,6 +383,19 @@ int flush_pending_invalidation(const Arena* ca, cudaStream_t st) {
   invalidate_survivors_kernel<<<1, 256, 0, st>>>(a->dev, a->pending_inval_row);
   a->pending_inval_row = -1;
   FDQL_CUDA(cudaGetLastError());
+  return FDQL_OK;
+}
+
+int check_packed_rows(const Arena* a, int32_t n_eps, const int32_t* ep_len, int64_t n_rows, cudaStream_t st) {
+  std::vector<int32_t> len(n_eps);
+  FDQL_CUDA(cudaMemcpyAsync(len.data(), ep_len, sizeof(int32_t) * n_eps, cudaMemcpyDeviceToHost, st));
+  FDQL_CUDA(cudaStreamSynchronize(st));
+  int64_t sum = 0;
+  for (int e = 0; e < n_eps; ++e) {
+    FDQL_REQUIRE(len[e] >= 1 && len[e] <= a->dev.capacity, "ep_len[%d] = %d is not in [1, capacity]", e, len[e]);
+    sum += len[e];
+  }
+  FDQL_REQUIRE(sum == n_rows, "n_rows = %lld but the episodes hold %lld rows", (long long)n_rows, (long long)sum);
   return FDQL_OK;
 }
 
@@ -757,8 +784,33 @@ int fdql_her_flush_episodes(fdql_arena* a, int32_t n_eps, const int64_t* src_beg
   if (rc) return rc;
   const int lpr = lanes_per_row(a->dev.wide[a->dev.wide_ag].vecs);
   const unsigned blocks = (unsigned)(((int64_t)n_eps * 32 + 255) / 256);
-  FDQL_DISPATCH_LPR(lpr, (her_flush_kernel<LPR><<<blocks, 256, 0, (cudaStream_t)stream>>>(
+  FDQL_DISPATCH_LPR(lpr, (her_flush_kernel<LPR, RewardSpec><<<blocks, 256, 0, (cudaStream_t)stream>>>(
                              a->dev, n_eps, src_begin, ep_len, dst_begin, goal_row, rs, gamma, with_returns)));
+  FDQL_CUDA(cudaGetLastError());
+  return FDQL_OK;
+}
+
+int fdql_her_flush_episodes_given(fdql_arena* a, int32_t n_eps, const int64_t* src_begin, const int32_t* ep_len,
+                                  const int64_t* dst_begin, const int64_t* goal_row, int64_t n_rows, const float* reward,
+                                  const uint8_t* done, const float* reward_dg, double gamma, int32_t with_returns, void* stream) {
+  FDQL_REQUIRE(a != nullptr && n_eps >= 0 && n_rows >= 0, "bad argument");
+  if (n_eps == 0) {
+    FDQL_REQUIRE(n_rows == 0, "n_rows = %lld but there are no episodes", (long long)n_rows);
+    return FDQL_OK;
+  }
+  FDQL_REQUIRE(src_begin && ep_len && dst_begin && goal_row, "null episode table");
+  FDQL_REQUIRE(reward && done && reward_dg, "null reward, done or reward_dg array");
+  FDQL_REQUIRE(a->dev.wide_ag >= 0 && a->dev.wide_dg >= 0, "hindsight flush needs achieved_goal and desired_goal keys");
+  FDQL_REQUIRE(a->dev.wide[a->dev.wide_ag].vecs <= 32, "goal wider than 128 floats is not supported");
+  int rc = check_packed_rows(a, n_eps, ep_len, n_rows, (cudaStream_t)stream);
+  if (rc) return rc;
+  rc = flush_pending_invalidation(a, (cudaStream_t)stream);
+  if (rc) return rc;
+  const GivenReward g{reward, done, reward_dg};
+  const int lpr = lanes_per_row(a->dev.wide[a->dev.wide_ag].vecs);
+  const unsigned blocks = (unsigned)(((int64_t)n_eps * 32 + 255) / 256);
+  FDQL_DISPATCH_LPR(lpr, (her_flush_kernel<LPR, GivenReward><<<blocks, 256, 0, (cudaStream_t)stream>>>(
+                             a->dev, n_eps, src_begin, ep_len, dst_begin, goal_row, g, gamma, with_returns)));
   FDQL_CUDA(cudaGetLastError());
   return FDQL_OK;
 }

@@ -6,6 +6,7 @@
 #include <string.h>
 
 #include <mutex>
+#include <type_traits>
 
 #include "../../include/fdql.h"
 
@@ -189,6 +190,29 @@ std::mutex& cursor_mutex();
 
 int upload_reward_spec(const Arena* a, int32_t op, const float* params_host, int32_t n_params, cudaStream_t st,
                        RewardSpec* out);
+
+// Reward source of the write-time flush kernels (her_flush_kernel, vmap_flush_kernel): either a RewardSpec, whose functor the kernel
+// evaluates on the goals in the ring, or a GivenReward, whose per-row results a caller computed beforehand and packed episode after
+// episode in the order of the episode table (fdql_her_flush_episodes_given, fdql_vmap_flush_episodes_given).
+struct GivenReward {
+  const float* reward;     // R(ag_i, goal): [n_rows] (hindsight flush) or [n_rows, V+1] (vmap fill)
+  const uint8_t* done;     // done of the same pairs, non-zero = done
+  const float* reward_dg;  // R(ag_i, dg_i) [n_rows] (hindsight flush; the vmap fill reads column V of `reward` instead)
+};
+template <class Reward>
+constexpr bool kGivenReward = std::is_same<Reward, GivenReward>::value;
+
+// First packed row of episode e in a GivenReward: the sum of ep_len[0 .. e), summed by the calling warp (all 32 lanes active).
+__device__ __forceinline__ int64_t packed_first_row(const int32_t* __restrict__ ep_len, int e) {
+  long long s = 0;
+  for (int i = threadIdx.x & 31; i < e; i += 32) s += ep_len[i];
+  for (int m = 16; m >= 1; m >>= 1) s += __shfl_xor_sync(kFull, s, m);
+  return s;
+}
+
+// Host check of a *_given call: reads the device table ep_len[n_eps] back (synchronising `st`) and requires every length in
+// [1, capacity] and their sum equal to n_rows, the rows of the packed arrays.
+int check_packed_rows(const Arena* a, int32_t n_eps, const int32_t* ep_len, int64_t n_rows, cudaStream_t st);
 
 }  // namespace fdql
 

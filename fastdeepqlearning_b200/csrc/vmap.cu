@@ -40,16 +40,22 @@ __device__ __forceinline__ void eval_row_thread(const RewardSpec& rs, const floa
   done = ok;
 }
 
-// mode bit 0: fill virtual_goals / virtual_rewards / virtual_dones (HindsightVmapWrite); bit 1: virtual_mc_return (NStepReturnVmap)
+// mode bit 0: fill virtual_goals / virtual_rewards / virtual_dones (HindsightVmapWrite); bit 1: virtual_mc_return (NStepReturnVmap).
+// Reward = RewardSpec evaluates R(ag, vg) and R(ag, dg) with the device functor; GivenReward loads them from the packed
+// [n_rows, V+1] grid, whose column V holds R(ag, dg) (common.cuh).
+template <class Reward>
 __global__ void __launch_bounds__(128) vmap_flush_kernel(ArenaDev A, VmapKeys K, int32_t n_eps, const int64_t* __restrict__ ep_begin,
                                                         const int32_t* __restrict__ ep_len, const int64_t* __restrict__ pick_rows,
-                                                        RewardSpec rs, double gamma, int mode, int done_quirk) {
+                                                        Reward rw, double gamma, int mode, int done_quirk) {
+  constexpr bool given = kGivenReward<Reward>;
   const int ep = blockIdx.x;
   if (ep >= n_eps) return;
   const int64_t s = ep_begin[ep];
   const int L = ep_len[ep];
   const int V = K.V, G = K.G, C1 = V + 1;
   if (mode & 1) {
+    int64_t p0 = 0;  // first packed row of this episode (GivenReward)
+    if constexpr (given) p0 = packed_first_row(ep_len, ep);
     const WideSlab AG = A.wide[A.wide_ag], DG = A.wide[A.wide_dg];
     const int64_t* picks = pick_rows + (int64_t)ep * V;
     for (int item = threadIdx.x; item < L * C1; item += blockDim.x) {
@@ -67,8 +73,16 @@ __global__ void __launch_bounds__(128) vmap_flush_kernel(ArenaDev A, VmapKeys K,
         goal = AG.base + picks[v] * (int64_t)AG.stride;
         float Rd, Rv;
         bool dd, dv;
-        eval_row_thread(rs, ag, dg, G, Rd, dd);
-        eval_row_thread(rs, ag, goal, G, Rv, dv);
+        if constexpr (given) {
+          const int64_t k = (p0 + j) * C1;
+          Rd = rw.reward[k + V];
+          dd = rw.done[k + V] != 0;
+          Rv = rw.reward[k + v];
+          dv = rw.done[k + v] != 0;
+        } else {
+          eval_row_thread(rw, ag, dg, G, Rd, dd);
+          eval_row_thread(rw, ag, goal, G, Rv, dv);
+        }
         vr = __fadd_rn(__fsub_rn(r, Rd), Rv);  // float32 like jax: (reward - desired_reward) + virtual_reward  (:34,39)
         vd = (done && !dd) || dv;              // (done and not desired_done) or virtual_done                 (:37,40)
       }
@@ -222,8 +236,38 @@ int fdql_vmap_flush_episodes(fdql_arena* a, int32_t n_eps, const int64_t* ep_beg
     if (rc) return rc;
   }
   if (mode & 2) FDQL_REQUIRE(key_returns >= 0, "the returns mode needs a virtual_mc_return key");
-  vmap_flush_kernel<<<(unsigned)n_eps, 128, 0, (cudaStream_t)stream>>>(a->dev, K, n_eps, ep_begin, ep_len, pick_rows, rs, gamma, mode,
-                                                                     done_quirk);
+  vmap_flush_kernel<RewardSpec><<<(unsigned)n_eps, 128, 0, (cudaStream_t)stream>>>(a->dev, K, n_eps, ep_begin, ep_len, pick_rows, rs,
+                                                                                 gamma, mode, done_quirk);
+  FDQL_CUDA(cudaGetLastError());
+  return FDQL_OK;
+}
+
+int fdql_vmap_flush_episodes_given(fdql_arena* a, int32_t n_eps, const int64_t* ep_begin, const int32_t* ep_len,
+                                   const int64_t* pick_rows, int32_t key_goals, int32_t key_rewards, int32_t key_dones,
+                                   int32_t key_returns, int64_t n_rows, const float* reward, const uint8_t* done, double gamma,
+                                   int32_t mode, int32_t done_quirk, void* stream) {
+  FDQL_REQUIRE(a != nullptr && n_eps >= 0 && n_rows >= 0, "bad argument");
+  FDQL_REQUIRE((mode & 1) != 0 && (mode & ~3) == 0, "mode: bit 0 (fill goals/rewards/dones from the given grid) must be set, bit 1 = returns");
+  if (n_eps == 0) {
+    FDQL_REQUIRE(n_rows == 0, "n_rows = %lld but there are no episodes", (long long)n_rows);
+    return FDQL_OK;
+  }
+  FDQL_REQUIRE(ep_begin != nullptr && ep_len != nullptr, "null episode table");
+  FDQL_REQUIRE(pick_rows != nullptr, "the fill mode needs the rows whose achieved_goal become the virtual goals");
+  FDQL_REQUIRE(reward != nullptr && done != nullptr, "null reward or done grid");
+  VmapKeys K;
+  int rc = vmap_keys(a, key_goals, key_rewards, key_dones, key_returns, &K);
+  if (rc) return rc;
+  FDQL_REQUIRE(a->dev.wide_ag >= 0 && a->dev.wide_dg >= 0 && a->dev.col_reward >= 0 && a->dev.col_task_done >= 0,
+               "the fill mode needs achieved_goal, desired_goal, reward and task_done keys");
+  FDQL_REQUIRE(a->dev.wide[a->dev.wide_ag].width == K.G && a->dev.wide[a->dev.wide_dg].width == K.G,
+               "goal width %d does not match virtual_goals (%d per goal)", a->dev.wide[a->dev.wide_ag].width, K.G);
+  if (mode & 2) FDQL_REQUIRE(key_returns >= 0, "the returns mode needs a virtual_mc_return key");
+  rc = check_packed_rows(a, n_eps, ep_len, n_rows, (cudaStream_t)stream);
+  if (rc) return rc;
+  const GivenReward g{reward, done, nullptr};
+  vmap_flush_kernel<GivenReward><<<(unsigned)n_eps, 128, 0, (cudaStream_t)stream>>>(a->dev, K, n_eps, ep_begin, ep_len, pick_rows, g,
+                                                                                  gamma, mode, done_quirk);
   FDQL_CUDA(cudaGetLastError());
   return FDQL_OK;
 }

@@ -123,6 +123,20 @@ int fdql_her_flush_episodes(fdql_arena* a, int32_t n_eps, const int64_t* src_beg
                             const int64_t* dst_begin, const int64_t* goal_row, int32_t reward_op,
                             const float* reward_params_host, int32_t n_params, double gamma, int32_t with_returns,
                             void* stream);
+/* fdql_her_flush_episodes with the rewards computed beforehand (for a reward function the functors cannot express, evaluated by the
+ * caller on the device before the call) instead of by a functor.  The episode arguments and the rows written are those of
+ * fdql_her_flush_episodes: desired_goal := achieved_goal[goal_row], reward := (r - R(ag, dg)) + R(ag, g*) in fp64 rounded to fp32,
+ * task_done := done(R(ag, g*)), episode_step re-based at every relabelled terminal (her.py:72-83), the extents of the copy, and
+ * mc_return over the whole real episode (quirk Q5).
+ * Packed layout: the n_rows = sum(ep_len) source rows episode after episode in the order of the episode table, each episode
+ * oldest row first, so that source row j of episode e is packed row sum(ep_len[0..e)) + j.  Device arrays of n_rows each:
+ *   reward[i], done[i]  R(ag_i, g*) of the row and its episode's goal g* = achieved_goal[goal_row[e]] (done: non-zero = done);
+ *   reward_dg[i]        R(ag_i, dg_i), the row's reward under its own desired_goal (the goal-agnostic term of her.py:65-68).
+ * Needs achieved_goal and desired_goal keys.  Reads ep_len back to the host to check sum(ep_len) == n_rows, so the call waits for the
+ * work already enqueued on `stream`. */
+int fdql_her_flush_episodes_given(fdql_arena* a, int32_t n_eps, const int64_t* src_begin, const int32_t* ep_len,
+                                  const int64_t* dst_begin, const int64_t* goal_row, int64_t n_rows, const float* reward,
+                                  const uint8_t* done, const float* reward_dg, double gamma, int32_t with_returns, void* stream);
 /* advance the cursor by n rows without writing them (their content is produced by fdql_her_flush_episodes) */
 int fdql_arena_reserve(fdql_arena* a, int64_t n_rows, int64_t* first_row);
 
@@ -153,6 +167,18 @@ int fdql_vmap_flush_episodes(fdql_arena* a, int32_t n_eps, const int64_t* ep_beg
                              int32_t key_goals, int32_t key_rewards, int32_t key_dones, int32_t key_returns, int32_t reward_op,
                              const float* reward_params_host, int32_t n_params, double gamma, int32_t mode, int32_t done_quirk,
                              void* stream);
+/* fdql_vmap_flush_episodes with the rewards computed beforehand instead of by a functor (see fdql_her_flush_episodes_given).  Mode bit
+ * 0 must be set; bit 1 and done_quirk act as above.  Packed layout: the n_rows = sum(ep_len) rows episode after episode in the order
+ * of the episode table, each oldest row first; reward and done are device grids [n_rows, V+1] (row-major; done: non-zero = done):
+ *   column v < V  R(ag_i, achieved_goal[pick_rows[e*V + v]]), the row under virtual goal v of its episode;
+ *   column V      R(ag_i, dg_i), the row under its own desired_goal (the term the virtual rewards and dones are rebased from).
+ * virtual_reward = (reward - column V) + column v in float32, virtual_done = (task_done and not done[V]) or done[v]; column V of
+ * the stored keys keeps the row's own reward and task_done as in fdql_vmap_flush_episodes.  Reads ep_len back to the host to check
+ * sum(ep_len) == n_rows, so the call waits for the work already enqueued on `stream`. */
+int fdql_vmap_flush_episodes_given(fdql_arena* a, int32_t n_eps, const int64_t* ep_begin, const int32_t* ep_len,
+                                   const int64_t* pick_rows, int32_t key_goals, int32_t key_rewards, int32_t key_dones,
+                                   int32_t key_returns, int64_t n_rows, const float* reward, const uint8_t* done, double gamma,
+                                   int32_t mode, int32_t done_quirk, void* stream);
 
 /* HindsightVmapRead.temporal_sample (franQ/Replay/wrappers/her_vmap.py:104-123) for windows (starts[b]+t) % len, t<T:
  * desired_goal [T,n,G] := virtual_goals[..., column, :], reward / task_done / mc_return [T,n,1] := the same column of
