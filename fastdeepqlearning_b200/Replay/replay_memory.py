@@ -23,6 +23,8 @@ from .. import _lib as L
 from .._lib import OversampleError, check
 from ..reward_ops import RewardOp, TorchReward, require_device_functor
 
+MAX_GOAL_WIDTH = 128  # widest achieved_goal / desired_goal the relabel kernels serve (include/fdql.h)
+
 
 def _locked(fn):
     """One writer thread (Runner._replay_handler) and the learner's reader thread share a ring in the reference without a lock
@@ -93,6 +95,11 @@ class ReplayMemory:
         self._widths = [int(widths[k]) for k in self._keys]
         self._shapes = dict(shapes or {k: (w,) for k, w in widths.items()})
         roles = [self._role_override.get(k, L.ROLE_BY_NAME.get(k, L.ROLE_NONE)) for k in self._keys]
+        for k, w, r in zip(self._keys, self._widths, roles):
+            if r == L.ROLE_ACHIEVED_GOAL and w > MAX_GOAL_WIDTH:
+                # every episode commit hashes the achieved goals with the relabel kernels' lane layout: refuse before a row is stored
+                # (a desired_goal alone is never evaluated; with an achieved_goal the arena requires both of one width)
+                raise ValueError(f"{k}: goal wider than {MAX_GOAL_WIDTH} floats is not supported (width {w})")
         n = len(self._keys)
         h = C.c_void_p()
         check(self._lib.fdql_arena_create(self._maxlen, n, (C.c_int32 * n)(*self._widths), (C.c_int32 * n)(*roles),

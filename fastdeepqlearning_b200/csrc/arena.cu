@@ -744,16 +744,16 @@ int fdql_commit_episodes(fdql_arena* a, int32_t n_eps, const int64_t* ep_begin, 
   FDQL_REQUIRE(a != nullptr && n_eps >= 0, "bad argument");
   if (n_eps == 0) return FDQL_OK;
   FDQL_REQUIRE(ep_begin != nullptr && ep_len != nullptr, "null episode table");
-  RewardSpec rs;
-  int rc = upload_reward_spec(a, reward_op, reward_params_host, n_params, (cudaStream_t)stream, &rs);
-  if (rc) return rc;
-  rc = flush_pending_invalidation(a, (cudaStream_t)stream);
-  if (rc) return rc;
   int lpr = 1;
   if (a->dev.wide_ag >= 0) {
     FDQL_REQUIRE(a->dev.wide[a->dev.wide_ag].vecs <= 32, "goal wider than 128 floats is not supported");
     lpr = lanes_per_row(a->dev.wide[a->dev.wide_ag].vecs);
   }
+  RewardSpec rs;
+  int rc = upload_reward_spec(a, reward_op, reward_params_host, n_params, (cudaStream_t)stream, &rs);
+  if (rc) return rc;
+  rc = flush_pending_invalidation(a, (cudaStream_t)stream);
+  if (rc) return rc;
   const unsigned blocks = (unsigned)(((int64_t)n_eps * 32 + 255) / 256);
   if (a->link_state == 0) {
     a->link_gamma = gamma;

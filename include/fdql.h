@@ -45,7 +45,9 @@ enum {
 };
 
 /* Device reward functors R(achieved_goal, goal) -> (reward, done); the enum-dispatched stand-in for the
- * Python callable HindsightNStepReplay receives (franQ/Replay/wrappers/her.py:13,62,67). */
+ * Python callable HindsightNStepReplay receives (franQ/Replay/wrappers/her.py:13,62,67).
+ * Goals (achieved_goal / desired_goal) of at most 128 floats are served: episode commits, hindsight flushes and the relabelling
+ * gather return FDQL_EINVAL ("goal wider than 128 floats is not supported") on a wider goal. */
 enum {
   FDQL_REWARD_NONE = 0,
   FDQL_REWARD_BITFLIP = 1,      /* franQ/Env/bitflip.py:143-152: all(ag==g) ? 0 : -1; done = reward==0          */

@@ -201,6 +201,17 @@ def make_reward_weighted_pnorm(weights, success_threshold, p=0.5):
     return f
 
 
+def fp32_reward(reward_fn):
+    """``reward_fn`` with its reward rounded to fp32 and its done left as the fp64 evaluation decided it: the form in which a
+    reward value reaches a float32 ring (the device functors evaluate in fp64 and store fp32, as the env's reward column is)."""
+
+    def f(ag, dg):
+        r, d = reward_fn(ag, dg)
+        return np.asarray(r, np.float64).astype(np.float32).astype(np.float64), d
+
+    return f
+
+
 REWARD_OPS = {"bitflip": reward_bitflip, "all_geq": reward_all_geq, "first_geq": reward_first_geq}
 
 
