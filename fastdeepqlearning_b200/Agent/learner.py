@@ -26,7 +26,9 @@ class LearnerConf(types.SimpleNamespace):
                  obs_keys=("obs_1d", "achieved_goal", "desired_goal"), use_bootstrap_minibatch_nstep=False, clip_grad_norm=None,
                  # prioritized replay (Schaul et al. 2016; not a reference mode): priority exponent, importance-sampling exponent annealed
                  # linearly from per_beta0 to 1 over per_beta_steps updates, priority floor, max / mean mix over a window (R2D2)
-                 use_prioritized_replay=False, per_alpha=0.6, per_beta0=0.4, per_beta_steps=100_000, per_eps=1e-6, per_eta=0.9)
+                 use_prioritized_replay=False, per_alpha=0.6, per_beta0=0.4, per_beta_steps=100_000, per_eps=1e-6, per_eta=0.9,
+                 # {key: uint8 / int8} keys the ring stores at one byte per element (image frames, bit-flip states); batches stay fp32
+                 replay_key_dtypes=None)
         d.update(kw)
         super().__init__(**d)
 

@@ -11,7 +11,9 @@ def make(conf, **kwargs):
     `kwargs["compute_reward"]` is a device reward functor (fastdeepqlearning_b200.RewardOp) or, for the write-time modes
     ("final", "random", "vmap"), a fastdeepqlearning_b200.TorchReward."""
     device = getattr(conf, "training_device", "cuda:0")
-    shards = [AsyncReplayMemory(int(conf.replay_size), conf.batch_size, conf.temporal_len, device=device)
+    # conf.replay_key_dtypes (optional): {key: uint8 / int8} keys stored at one byte per element, sampled as fp32 (ReplayMemory)
+    shards = [AsyncReplayMemory(int(conf.replay_size), conf.batch_size, conf.temporal_len, device=device,
+                                key_dtypes=getattr(conf, "replay_key_dtypes", None))
               for _ in range(conf.num_instances)]
     write_heads = read_heads = shards
     her_mode = getattr(conf, "her_mode", "final")

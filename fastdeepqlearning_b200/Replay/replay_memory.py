@@ -3,7 +3,9 @@
 Same constructor, same duck type (`add`, `sample`, `temporal_sample`, `__getitem__`, `__len__`), same cursor
 arithmetic (quirk Q1: the length saturates at maxlen-1) and the same `OversampleError`.  Differences, all on purpose:
   * storage is fp32 structure-of-arrays slabs in HBM (the dtype franQ's TorchDataLoader casts every key to,
-    torch_dataloader.py:36); values must be fp32-representable;
+    torch_dataloader.py:36); values must be fp32-representable.  A key declared in `key_dtypes` as uint8 or int8 (observations,
+    actions: role-less keys of width >= 2) is stored at one byte per element instead, as franQ's ring keeps a numpy array's dtype,
+    and every sample still hands it out as exact fp32 values;
   * samples are CUDA tensors `[T, B, w]`, not numpy arrays, so TorchDataLoader becomes a pass-through;
   * `add` stages rows in pinned host memory and moves them in batches; any read flushes first;
   * rows of finished episodes carry their episode extents so that sampled windows can be hindsight-relabelled
@@ -24,6 +26,50 @@ from .._lib import OversampleError, check
 from ..reward_ops import RewardOp, TorchReward, require_device_functor
 
 MAX_GOAL_WIDTH = 128  # widest achieved_goal / desired_goal the relabel kernels serve (include/fdql.h)
+# storage types of narrow keys (fdql_arena_create_typed): torch dtype, C code, numpy dtype, inclusive value range
+_NARROW = {torch.uint8: (L.DTYPE_U8, np.uint8, 0, 255), torch.int8: (L.DTYPE_I8, np.int8, -128, 127)}
+
+
+def _narrow_dtype(k, dt):
+    """torch.uint8 / torch.int8 from a torch or numpy dtype (or its name); ValueError for anything else."""
+    if not isinstance(dt, torch.dtype):
+        try:
+            dt = {np.dtype(np.uint8): torch.uint8, np.dtype(np.int8): torch.int8}.get(np.dtype(dt))
+        except TypeError:
+            dt = None
+    if dt not in _NARROW:
+        raise ValueError(f"key_dtypes[{k!r}]: only uint8 and int8 keys can be stored narrow, got {dt}")
+    return dt
+
+
+def _exact_narrow(k, v, dt):
+    """`v` (array-like or torch tensor, any device) as `dt` when every value is an integer the type holds exactly; ValueError otherwise
+    (never wraps: 256 or -1 for uint8, 0.5 and NaN are refused)."""
+    lo, hi = _NARROW[dt][2], _NARROW[dt][3]
+    bad = f"{k}: values outside the {dt} range [{lo}, {hi}] or not integers; a narrow key stores them exactly"
+    if isinstance(v, torch.Tensor):
+        if v.dtype == dt or v.dtype == torch.bool:
+            return v.to(dt)
+        if v.is_complex():
+            raise ValueError(f"{k}: {v.dtype} values cannot be stored in a {dt} key")
+        ok = (v >= lo) & (v <= hi)  # NaN fails both
+        if v.dtype.is_floating_point:
+            ok &= v == torch.trunc(v)
+        if v.numel() and not bool(ok.all()):
+            raise ValueError(bad)
+        return v.to(dt)
+    a = np.asarray(v)
+    if a.dtype == _NARROW[dt][1] or a.dtype.kind == "b":
+        return a.astype(_NARROW[dt][1], copy=False)
+    if a.dtype.kind not in "iuf":
+        raise ValueError(f"{k}: {a.dtype} values cannot be stored in a {dt} key")
+    with np.errstate(invalid="ignore"):
+        ok = (a >= lo) & (a <= hi)  # NaN fails both
+        if a.dtype.kind == "f":
+            ok &= a == np.trunc(a)
+    if a.size and not bool(np.all(ok)):
+        raise ValueError(bad)
+    return a.astype(_NARROW[dt][1])
 
 
 def _locked(fn):
@@ -45,13 +91,15 @@ def _stream_ptr(device):
 class _DevView:
     """__cuda_array_interface__ carrier for zero-copy torch views of arena slabs."""
 
-    def __init__(self, ptr, shape, strides_bytes):
-        self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": "<f4", "data": (int(ptr), False), "version": 3,
+    def __init__(self, ptr, shape, strides_bytes, typestr="<f4"):
+        self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": typestr, "data": (int(ptr), False), "version": 3,
                                          "strides": tuple(strides_bytes)}
 
 
 class ReplayMemory:
-    def __init__(self, maxlen, batch_size, temporal_len, device="cuda:0", stage_rows=1024, roles=None, **kwargs):
+    def __init__(self, maxlen, batch_size, temporal_len, device="cuda:0", stage_rows=1024, roles=None, key_dtypes=None, **kwargs):
+        """`key_dtypes` ({key: torch.uint8 / torch.int8 or the numpy dtype}) stores those keys at one byte per element (image frames,
+        bit-flip states); they must be role-less keys of width >= 2.  Checked when the first row arrives."""
         self._batch_size, self._temporal_len, self._maxlen = batch_size, temporal_len, int(maxlen)
         self.batch_size = batch_size
         self._top, self._curr_len = 0, 0
@@ -65,6 +113,8 @@ class ReplayMemory:
         self._widths: T.List[int] = []
         self._shapes: T.Dict[str, tuple] = {}
         self._role_override = dict(roles or {})
+        self._key_dtypes_conf = dict(key_dtypes or {})
+        self._narrow: T.Dict[str, torch.dtype] = {}  # key -> torch.uint8 / torch.int8 once the arena exists
         self._stage_rows = max(1, min(int(stage_rows), self._maxlen))  # a flush never carries more rows than the ring holds
         self._stage = None       # two pinned host blocks [stage_rows, row_floats]: add() packs rows into one while the other drains
         self._stage_np = None    # per block: key -> numpy view [stage_rows, width] into the block
@@ -100,20 +150,39 @@ class ReplayMemory:
                 # every episode commit hashes the achieved goals with the relabel kernels' lane layout: refuse before a row is stored
                 # (a desired_goal alone is never evaluated; with an achieved_goal the arena requires both of one width)
                 raise ValueError(f"{k}: goal wider than {MAX_GOAL_WIDTH} floats is not supported (width {w})")
+        narrow = {}
+        for k, dt in self._key_dtypes_conf.items():
+            if k not in self._keys:
+                raise ValueError(f"key_dtypes names {k!r}, which is not a key of the rows ({self._keys})")
+            if k in self.VMAP_KEYS:
+                raise ValueError(f"key_dtypes: {k!r} is a virtual key of the vmap hindsight mode and stays fp32")
+            i = self._keys.index(k)
+            if roles[i] != L.ROLE_NONE or self._widths[i] < 2:
+                raise ValueError(f"key_dtypes: {k!r} is a scalar or role key (reward, dones, steps, returns, goals) and stays fp32; "
+                                 f"only role-less keys of width >= 2 can be stored narrow")
+            narrow[k] = _narrow_dtype(k, dt)
         n = len(self._keys)
         h = C.c_void_p()
-        check(self._lib.fdql_arena_create(self._maxlen, n, (C.c_int32 * n)(*self._widths), (C.c_int32 * n)(*roles),
-                                          self.device.index or 0, C.byref(h)))
+        dtypes = [_NARROW[narrow[k]][0] if k in narrow else L.DTYPE_F32 for k in self._keys]
+        check(self._lib.fdql_arena_create_typed(self._maxlen, n, (C.c_int32 * n)(*self._widths), (C.c_int32 * n)(*roles),
+                                                (C.c_int32 * n)(*dtypes), self.device.index or 0, C.byref(h)))
         self._h = h
-        # packed staging: every key of a row side by side, offsets and row size multiples of 4 floats (128-bit path of the append kernel)
+        self._narrow = narrow
+        # packed staging: every key of a row side by side, offsets and row size multiples of 4 floats (128-bit path of the append kernel);
+        # a narrow key's region holds its raw bytes, ceil(w / 16) * 4 floats wide
         self._key_off, off = [], 0
-        for w in self._widths:
+        for k, w in zip(self._keys, self._widths):
             self._key_off.append(off)
-            off += (w + 3) // 4 * 4
+            off += (w + 15) // 16 * 4 if k in narrow else (w + 3) // 4 * 4
         self._row_floats = off
         self._key_off_c = (C.c_int32 * n)(*self._key_off)
         self._stage = [torch.zeros((self._stage_rows, self._row_floats), dtype=torch.float32).pin_memory() for _ in range(2)]
-        self._stage_np = [{k: blk.numpy()[:, o:o + w] for k, o, w in zip(self._keys, self._key_off, self._widths)} for blk in self._stage]
+
+        def view(blk, k, o, w):
+            if k not in narrow:
+                return blk.numpy()[:, o:o + w]
+            return blk.numpy()[:, o:o + (w + 15) // 16 * 4].view(_NARROW[narrow[k]][1])[:, :w]
+        self._stage_np = [{k: view(blk, k, o, w) for k, o, w in zip(self._keys, self._key_off, self._widths)} for blk in self._stage]
         self._scalar_key = {k: (w == 1) for k, w in zip(self._keys, self._widths)}
         if self._per_conf is not None:
             self._create_per()
@@ -157,6 +226,8 @@ class ReplayMemory:
                         "Anything thats not a numpy array must be representable as a float32 for numeric stability"
                     widths[k], shapes[k] = 1, (1,)
             self._jit_initialize(widths, shapes)
+        if self._narrow:  # checked whole before anything is staged
+            experience_dict = {k: _exact_narrow(k, v, self._narrow[k]) if k in self._narrow else v for k, v in experience_dict.items()}
         i = self._n_staged
         views = self._stage_np[self._stage_cur]
         for k, v in experience_dict.items():
@@ -226,8 +297,13 @@ class ReplayMemory:
         n = int(first.shape[0])
         self.ensure_schema(cols)
         self.flush()
+        narrow = {k: _exact_narrow(k, cols[k] if isinstance(cols[k], torch.Tensor) else np.asarray(cols[k]), dt)
+                  for k, dt in self._narrow.items()}
         dev = []
         for k, w in zip(self._keys, self._widths):
+            if k in narrow:
+                dev.append(torch.as_tensor(narrow[k]).to(device=self.device, non_blocking=True).reshape(n, w).contiguous())
+                continue
             t = torch.as_tensor(cols[k])
             t = t.to(device=self.device, dtype=torch.float32, non_blocking=True).reshape(n, w).contiguous()
             if self.squash_rewards and k == "reward":  # squash_rewards.py:5-7 in fp64 like numpy on the Python float, fp32 store
@@ -537,7 +613,8 @@ class ReplayMemory:
                 "reward_op": self._reward_op_state(),
                 "memory": {k: v.cpu().clone() for k, v in self.memory.items()}, "ep_start": es.cpu().clone(), "ep_end": ee.cpu().clone(),
                 "scan": self._meta_rows(2).view(torch.int32).cpu().clone(), "links": self._meta_rows(3).view(torch.int32).cpu().clone(),
-                "per": self._per_state()}
+                "per": self._per_state(),
+                **({"dtypes": {k: str(dt).replace("torch.", "") for k, dt in self._narrow.items()}} if self._narrow else {})}
 
     def _reward_op_state(self):
         """(op, params) of a RewardOp; "torch" for a TorchReward, whose function is not pickled (set it again before restoring)."""
@@ -563,11 +640,12 @@ class ReplayMemory:
         if sd["reward_op"] == "torch" and not isinstance(self.reward_op, TorchReward):
             raise ValueError("the snapshot's reward is a TorchReward, whose function a snapshot does not carry: call "
                              "set_reward_op(TorchReward(fn)) (or build the ring through its hindsight wrapper) before load_state_dict")
+        self._key_dtypes_conf = dict(sd.get("dtypes", {}))  # a snapshot without the entry is all fp32
         self._jit_initialize(dict(zip(sd["keys"], sd["widths"])), sd["shapes"])
         self.gamma = float(sd["gamma"])
         if sd["reward_op"] is not None and sd["reward_op"] != "torch":
             self.reward_op = RewardOp(sd["reward_op"][0], sd["reward_op"][1] or ())
-        dev = [sd["memory"][k].to(self.device, dtype=torch.float32).reshape(self._maxlen, w).contiguous()
+        dev = [sd["memory"][k].to(self.device, dtype=self._narrow.get(k, torch.float32)).reshape(self._maxlen, w).contiguous()
                for k, w in zip(self._keys, self._widths)]
         check(self._lib.fdql_arena_append(self._h, self._maxlen, L.ptr_array([t.data_ptr() for t in dev]), _stream_ptr(self.device)))
         check(self._lib.fdql_arena_set_cursor(self._h, int(sd["top"]), int(sd["len"])))
@@ -601,11 +679,23 @@ class ReplayMemory:
         return list(self._keys)
 
     @property
+    def key_dtypes(self) -> T.Dict[str, torch.dtype]:
+        """Storage type of every key: torch.float32, or torch.uint8 / torch.int8 for narrow keys."""
+        return {k: self._narrow.get(k, torch.float32) for k in self._keys}
+
+    @property
     def memory(self) -> T.Dict[str, torch.Tensor]:
-        """Zero-copy strided views of the arena slabs, `memory[k]` is [maxlen, w] like the reference's numpy dict."""
+        """Zero-copy strided views of the arena slabs, `memory[k]` is [maxlen, w] like the reference's numpy dict (uint8 / int8 for
+        narrow keys)."""
         self.flush()
         out = {}
         for i, (k, w) in enumerate(zip(self._keys, self._widths)):
+            if k in self._narrow:
+                base, stride, dt = C.c_void_p(), C.c_int64(), C.c_int32()
+                check(self._lib.fdql_arena_narrow_view(self._h, i, C.byref(base), C.byref(stride), C.byref(dt)))
+                out[k] = torch.as_tensor(_DevView(base.value, (self._maxlen, w), (stride.value, 1),
+                                                  "|u1" if self._narrow[k] == torch.uint8 else "|i1"), device=self.device)
+                continue
             base, stride, col = C.c_void_p(), C.c_int64(), C.c_int32()
             check(self._lib.fdql_arena_key_view(self._h, i, C.byref(base), C.byref(stride), C.byref(col)))
             out[k] = torch.as_tensor(_DevView(base.value + 4 * col.value, (self._maxlen, w), (4 * stride.value, 4)),

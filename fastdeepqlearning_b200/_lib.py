@@ -23,6 +23,7 @@ REWARD_NONE, REWARD_BITFLIP, REWARD_ALL_GEQ, REWARD_FIRST_GEQ, REWARD_WEIGHTED_P
 GOAL_FINAL, GOAL_RANDOM, GOAL_FUTURE = range(3)
 OPT_EXACT_EPISODE_STEP, OPT_EMIT_LEARNER_AUX, OPT_CORESIDENT = 1, 2, 4
 APPEND_SQUASH_REWARDS = 1
+DTYPE_F32, DTYPE_U8, DTYPE_I8 = 0, 1, 2  # storage types of fdql_arena_create_typed (uint8 / int8: "narrow" keys)
 
 
 class FdqlError(RuntimeError):
@@ -44,6 +45,8 @@ _SIGNATURES = {
     "fdql_last_error": (C.c_char_p, []),
     "fdql_version": (C.c_int, []),
     "fdql_arena_create": (C.c_int, [_i64, _i32, C.POINTER(_i32), C.POINTER(_i32), _i32, C.POINTER(_p)]),
+    "fdql_arena_create_typed": (C.c_int, [_i64, _i32, C.POINTER(_i32), C.POINTER(_i32), C.POINTER(_i32), _i32, C.POINTER(_p)]),
+    "fdql_arena_narrow_view": (C.c_int, [_p, _i32, C.POINTER(_p), C.POINTER(_i64), C.POINTER(_i32)]),
     "fdql_arena_destroy": (C.c_int, [_p]),
     "fdql_arena_info": (C.c_int, [_p, C.POINTER(_i64), C.POINTER(_i64), C.POINTER(_i64), C.POINTER(_i64)]),
     "fdql_arena_set_cursor": (C.c_int, [_p, _i64, _i64]),

@@ -450,15 +450,27 @@ int fdql_version(void) { return 100; }
 
 int fdql_arena_create(int64_t capacity, int32_t n_keys, const int32_t* widths, const int32_t* roles, int32_t device,
                       fdql_arena** out) {
+  return fdql_arena_create_typed(capacity, n_keys, widths, roles, nullptr, device, out);
+}
+
+int fdql_arena_create_typed(int64_t capacity, int32_t n_keys, const int32_t* widths, const int32_t* roles, const int32_t* dtypes,
+                            int32_t device, fdql_arena** out) {
   FDQL_REQUIRE(out != nullptr && widths != nullptr, "null argument");
   FDQL_REQUIRE(capacity >= 2 && capacity < (1ll << 31), "capacity must be in [2, 2^31)");
   FDQL_REQUIRE(n_keys >= 1 && n_keys <= FDQL_MAX_KEYS, "n_keys must be in [1, %d]", FDQL_MAX_KEYS);
+  for (int k = 0; k < n_keys && dtypes != nullptr; ++k) {
+    const int dt = dtypes[k], role = roles ? roles[k] : FDQL_ROLE_NONE;
+    FDQL_REQUIRE(dt == FDQL_DTYPE_F32 || dt == FDQL_DTYPE_U8 || dt == FDQL_DTYPE_I8, "key %d: unknown dtype %d", k, dt);
+    FDQL_REQUIRE(dt == FDQL_DTYPE_F32 || (role == FDQL_ROLE_NONE && widths[k] >= 2),
+                 "key %d: a uint8 / int8 key needs role NONE and width >= 2 (role %d, width %d)", k, role, widths[k]);
+  }
   FDQL_CUDA(cudaSetDevice(device));
   fdql_arena* a = new fdql_arena();
   memset(static_cast<Arena*>(a), 0, sizeof(Arena));
   a->n_keys = n_keys;
   a->device = device;
   a->pending_inval_row = -1;
+  a->narrow.capacity = capacity;
   ArenaDev& D = a->dev;
   D.capacity = capacity;
   D.col_reward = D.col_task_done = D.col_ep_done = D.col_ep_step = D.col_mc_return = -1;
@@ -472,9 +484,16 @@ int fdql_arena_create(int64_t capacity, int32_t n_keys, const int32_t* widths, c
     }
     a->widths[k] = w;
     a->roles[k] = role;
-    a->key_wide[k] = a->key_col[k] = -1;
+    a->key_wide[k] = a->key_col[k] = a->key_narrow[k] = -1;
     const bool goal = role == FDQL_ROLE_ACHIEVED_GOAL || role == FDQL_ROLE_DESIRED_GOAL;
-    if (w == 1 && !goal) {
+    if (dtypes != nullptr && dtypes[k] != FDQL_DTYPE_F32) {
+      NarrowSlab& S = a->narrow.s[a->narrow.n];
+      S.width = w;
+      S.stride = (w + 15) / 16 * 16;
+      S.dtype = dtypes[k];
+      S.key = k;
+      a->key_narrow[k] = a->narrow.n++;
+    } else if (w == 1 && !goal) {
       const int c = D.n_scal++;
       D.scal_key[c] = k;
       a->key_col[k] = c;
@@ -512,6 +531,8 @@ int fdql_arena_create(int64_t capacity, int32_t n_keys, const int32_t* widths, c
   };
   bool ok = true;
   for (int s = 0; s < D.n_wide && ok; ++s) ok = alloc(&D.wide[s].base, (size_t)capacity * D.wide[s].stride);
+  for (int s = 0; s < a->narrow.n && ok; ++s)
+    ok = alloc(reinterpret_cast<float**>(&a->narrow.s[s].base), (size_t)capacity * a->narrow.s[s].stride / sizeof(float));
   ok = ok && alloc(&D.rec, (size_t)capacity * D.rec_stride);
   ok = ok && alloc(reinterpret_cast<float**>(&D.scan), (size_t)capacity * 4);
   ok = ok && alloc(reinterpret_cast<float**>(&D.link), (size_t)capacity * 4);
@@ -534,6 +555,8 @@ int fdql_arena_destroy(fdql_arena* a) {
   if (!a) return FDQL_OK;
   for (int s = 0; s < a->dev.n_wide; ++s)
     if (a->dev.wide[s].base) cudaFree(a->dev.wide[s].base);
+  for (int s = 0; s < a->narrow.n; ++s)
+    if (a->narrow.s[s].base) cudaFree(a->narrow.s[s].base);
   if (a->dev.rec) cudaFree(a->dev.rec);
   if (a->dev.scan) cudaFree(a->dev.scan);
   if (a->dev.link) cudaFree(a->dev.link);
@@ -588,6 +611,7 @@ int fdql_arena_set_cursor(fdql_arena* a, int64_t top, int64_t len) {
 
 int fdql_arena_key_view(const fdql_arena* a, int32_t key, float** base, int64_t* row_stride, int32_t* col) {
   FDQL_REQUIRE(a != nullptr && key >= 0 && key < a->n_keys, "bad key");
+  FDQL_REQUIRE(a->key_narrow[key] < 0, "key %d is stored as uint8 / int8: use fdql_arena_narrow_view", key);
   if (a->key_wide[key] >= 0) {
     const WideSlab& W = a->dev.wide[a->key_wide[key]];
     *base = W.base;
@@ -598,6 +622,17 @@ int fdql_arena_key_view(const fdql_arena* a, int32_t key, float** base, int64_t*
     *row_stride = a->dev.rec_stride;
     *col = a->key_col[key];
   }
+  return FDQL_OK;
+}
+
+int fdql_arena_narrow_view(const fdql_arena* a, int32_t key, void** base, int64_t* row_stride_bytes, int32_t* dtype) {
+  FDQL_REQUIRE(a != nullptr && key >= 0 && key < a->n_keys, "bad key");
+  FDQL_REQUIRE(base != nullptr && row_stride_bytes != nullptr && dtype != nullptr, "null argument");
+  FDQL_REQUIRE(a->key_narrow[key] >= 0, "key %d is stored as fp32: use fdql_arena_key_view", key);
+  const NarrowSlab& S = a->narrow.s[a->key_narrow[key]];
+  *base = S.base;
+  *row_stride_bytes = S.stride;
+  *dtype = S.dtype;
   return FDQL_OK;
 }
 
@@ -650,6 +685,11 @@ int fdql_arena_append(fdql_arena* a, int64_t n_rows, const float* const* src, vo
   { int rc = flush_pending_invalidation(a, (cudaStream_t)stream); if (rc) return rc; }
   append_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(a->dev, sp, n_rows, a->top, a->append_src_stride, a->append_squash);
   FDQL_CUDA(cudaGetLastError());
+  {
+    const int rc = launch_narrow_append(a, n_rows, reinterpret_cast<const void* const*>(src), 4 * (int64_t)a->append_src_stride, a->top,
+                                        (cudaStream_t)stream);
+    if (rc) return rc;
+  }
   advance_cursor(a, n_rows);
   return FDQL_OK;
 }
@@ -660,8 +700,11 @@ int fdql_arena_append_packed_host(fdql_arena* a, int64_t n_rows, const float* pa
   FDQL_REQUIRE(n_rows >= 0 && n_rows <= a->dev.capacity, "n_rows must be in [0, capacity]");
   FDQL_REQUIRE(row_floats >= 1, "bad row size");
   if (n_rows == 0) return FDQL_OK;
-  for (int k = 0; k < a->n_keys; ++k)
-    FDQL_REQUIRE(key_offsets_host[k] >= 0 && key_offsets_host[k] + a->widths[k] <= row_floats, "key %d does not fit the packed row", k);
+  for (int k = 0; k < a->n_keys; ++k) {
+    // a narrow key's region holds its raw bytes, padded to 16: ceil(width / 16) * 4 floats
+    const int region = a->key_narrow[k] >= 0 ? (a->widths[k] + 15) / 16 * 4 : a->widths[k];
+    FDQL_REQUIRE(key_offsets_host[k] >= 0 && key_offsets_host[k] + region <= row_floats, "key %d does not fit the packed row", k);
+  }
   if (flags & FDQL_APPEND_SQUASH_REWARDS) FDQL_REQUIRE(a->dev.col_reward >= 0, "squashed rewards need a reward key");
   const size_t need = (size_t)n_rows * row_floats * sizeof(float);
   if (need > a->stage_bytes) {
@@ -689,7 +732,8 @@ int fdql_arena_append_host(fdql_arena* a, int64_t n_rows, const float* const* sr
   FDQL_REQUIRE(n_rows >= 0 && n_rows <= a->dev.capacity, "n_rows must be in [0, capacity]");
   if (n_rows == 0) return FDQL_OK;
   size_t need = 0;
-  for (int k = 0; k < a->n_keys; ++k) need += ((size_t)n_rows * a->widths[k] * sizeof(float) + 255) / 256 * 256;
+  auto key_bytes = [&](int k) { return (size_t)n_rows * a->widths[k] * (a->key_narrow[k] >= 0 ? 1 : sizeof(float)); };
+  for (int k = 0; k < a->n_keys; ++k) need += (key_bytes(k) + 255) / 256 * 256;
   if (need > a->stage_bytes) {
     FDQL_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
     if (a->stage_dev) cudaFree(a->stage_dev);
@@ -701,7 +745,7 @@ int fdql_arena_append_host(fdql_arena* a, int64_t n_rows, const float* const* sr
   const float* dev_ptrs[FDQL_MAX_KEYS];
   size_t off = 0;
   for (int k = 0; k < a->n_keys; ++k) {
-    const size_t b = (size_t)n_rows * a->widths[k] * sizeof(float);
+    const size_t b = key_bytes(k);
     float* d = reinterpret_cast<float*>(static_cast<char*>(a->stage_dev) + off);
     FDQL_CUDA(cudaMemcpyAsync(d, src_host[k], b, cudaMemcpyHostToDevice, (cudaStream_t)stream));
     dev_ptrs[k] = d;
@@ -717,7 +761,7 @@ int fdql_q3_duplicate(fdql_arena* a, int64_t src_row, int32_t n_step, int64_t ds
   { int rc = flush_pending_invalidation(a, (cudaStream_t)stream); if (rc) return rc; }
   q3_duplicate_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(a->dev, src_row, n_step, dst_row, gamma);
   FDQL_CUDA(cudaGetLastError());
-  return FDQL_OK;
+  return launch_narrow_copy(a, 1, nullptr, nullptr, nullptr, src_row, dst_row, (cudaStream_t)stream);
 }
 
 int fdql_arena_reserve(fdql_arena* a, int64_t n_rows, int64_t* first_row) {
@@ -787,7 +831,7 @@ int fdql_her_flush_episodes(fdql_arena* a, int32_t n_eps, const int64_t* src_beg
   FDQL_DISPATCH_LPR(lpr, (her_flush_kernel<LPR, RewardSpec><<<blocks, 256, 0, (cudaStream_t)stream>>>(
                              a->dev, n_eps, src_begin, ep_len, dst_begin, goal_row, rs, gamma, with_returns)));
   FDQL_CUDA(cudaGetLastError());
-  return FDQL_OK;
+  return launch_narrow_copy(a, n_eps, src_begin, ep_len, dst_begin, 0, 0, (cudaStream_t)stream);
 }
 
 int fdql_her_flush_episodes_given(fdql_arena* a, int32_t n_eps, const int64_t* src_begin, const int32_t* ep_len,
@@ -812,7 +856,7 @@ int fdql_her_flush_episodes_given(fdql_arena* a, int32_t n_eps, const int64_t* s
   FDQL_DISPATCH_LPR(lpr, (her_flush_kernel<LPR, GivenReward><<<blocks, 256, 0, (cudaStream_t)stream>>>(
                              a->dev, n_eps, src_begin, ep_len, dst_begin, goal_row, g, gamma, with_returns)));
   FDQL_CUDA(cudaGetLastError());
-  return FDQL_OK;
+  return launch_narrow_copy(a, n_eps, src_begin, ep_len, dst_begin, 0, 0, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -123,6 +123,13 @@ __device__ __forceinline__ int64_t ring_row(int64_t base, int64_t off, int64_t c
   int64_t r = base + off;
   return r >= cap ? r - cap : r;
 }
+// Row mapping of the window gathers (replay_memory.py:65): window start s is reduced modulo len, then row t of the window is
+// ring_row(window_start(s, len), t, len) (t < T <= len, so one wrap).  The descriptor-walking gather, the window setup of the tile /
+// lean / fused gathers and the narrow gather use these two; the warp-per-window fast kernel spells out the same arithmetic.
+__device__ __forceinline__ int64_t window_start(int64_t s, int64_t len) {
+  if (s >= len) s %= len;
+  return s;
+}
 
 __device__ __forceinline__ double shfl_down_f64(double v, int d) {
   int lo = __double2loint(v), hi = __double2hiint(v);
@@ -148,6 +155,22 @@ __device__ __forceinline__ double shfl_up_f64(double v, int d) {
   hi = __shfl_up_sync(kFull, hi, d);
   return __hiloint2double(hi, lo);
 }
+
+// Narrow keys (uint8 / int8, role NONE, width >= 2): one byte per element, [capacity, stride] bytes with stride = width rounded up to
+// 16 so that every row starts 16B-aligned.  They live in the host-side Arena only, never in ArenaDev::wide[]: the fp32 kernels do not
+// see them, and only the narrow kernels (narrow.cu) read or write them.
+struct NarrowSlab {
+  uint8_t* base;
+  int32_t stride;  // bytes, multiple of 16
+  int32_t width;   // elements
+  int32_t dtype;   // FDQL_DTYPE_U8 or FDQL_DTYPE_I8
+  int32_t key;     // caller's key index
+};
+struct NarrowSet {
+  int64_t capacity;
+  int32_t n;
+  NarrowSlab s[FDQL_MAX_KEYS];
+};
 
 // host-side view of an arena (definition shared by the translation units)
 struct Arena {
@@ -182,6 +205,9 @@ struct Arena {
   ::fdql_per* per;
   int64_t per_pending[4][2];
   int32_t n_per_pending;
+  // narrow keys (see NarrowSlab): narrow.s[key_narrow[k]] for key k, or key_narrow[k] = -1
+  NarrowSet narrow;
+  int32_t key_narrow[FDQL_MAX_KEYS];
 };
 
 int flush_pending_invalidation(const Arena* a, cudaStream_t st);
@@ -244,3 +270,16 @@ int launch_gather(const fdql_arena* a, int64_t n, int64_t b_begin, int64_t b_end
 }
 
 struct fdql_arena : fdql::Arena {};
+
+namespace fdql {
+// narrow.cu: the narrow-key halves of the gathers, the row copies and the append.  Each is a no-op on an arena without narrow keys.
+// Window rows as launch_gather: out[key] [T, n, width] fp32 for windows b_begin .. b_end of starts (NULL out[key]: key skipped).
+int launch_narrow_gather(const Arena* a, int64_t n, int64_t b_begin, int64_t b_end, int32_t T, int64_t len, const int64_t* starts,
+                         float* const* out, cudaStream_t st);
+// rows src_begin[e] + j -> dst_begin[e] + j (mod capacity), j < ep_len[e], e < n_eps (device tables); with src_begin == NULL one row
+// src_row -> dst_row
+int launch_narrow_copy(const Arena* a, int32_t n_eps, const int64_t* src_begin, const int32_t* ep_len, const int64_t* dst_begin,
+                       int64_t src_row, int64_t dst_row, cudaStream_t st);
+// n_rows rows from src[key] (device, row r at byte r * src_row_bytes, 0: dense [n_rows, width]) to ring rows top, top + 1, ...
+int launch_narrow_append(const Arena* a, int64_t n_rows, const void* const* src, int64_t src_row_bytes, int64_t top, cudaStream_t st);
+}  // namespace fdql

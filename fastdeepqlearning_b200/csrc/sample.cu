@@ -175,7 +175,7 @@ __global__ void __launch_bounds__(256) sample_gather_kernel(const __grid_constan
 
   for (int64_t b = g.b_begin + (int64_t)blockIdx.x * (blockDim.x >> 5) + wib; b < g.b_end; b += nwarps) {
     int64_t s = __ldg(g.starts + b);
-    if (s >= g.len) s %= g.len;
+    s = window_start(s, g.len);
 
     // ---- relabel set-up: episode extents of the start row, goal vector --------------------------
     bool relabel = false;
@@ -205,8 +205,7 @@ __global__ void __launch_bounds__(256) sample_gather_kernel(const __grid_constan
       const int items = T * W.vecs;
       for (int i = lane; i < items; i += 32) {
         const int t = i / W.vecs, v = i - t * W.vecs;
-        int64_t row = s + t;
-        if (row >= g.len) row -= g.len;
+        const int64_t row = ring_row(s, t, g.len);
         const float* src = (is_dg && t <= tail_last) ? S.base + grow * (int64_t)S.stride : W.base + row * (int64_t)W.stride;
         const float4 x = ldg4(src + 4 * v);
         float* dst = o + ((int64_t)t * g.n + b) * W.width + 4 * v;
@@ -278,8 +277,7 @@ __global__ void __launch_bounds__(256) sample_gather_kernel(const __grid_constan
     for (int tb = 0; tb < T; tb += 32) {
       const int t = tb + lane;
       const bool valid = t < T;
-      int64_t row = s + (valid ? t : 0);
-      if (row >= g.len) row -= g.len;
+      const int64_t row = ring_row(s, (valid ? t : 0), g.len);
       const float* rec = A.rec + row * (int64_t)A.rec_stride;
       const bool in_ep = RELABEL && relabel && valid && t <= tail_last;
       float v_step = 0.f, v_done = 0.f;
@@ -978,7 +976,7 @@ __device__ __forceinline__ void window_scalar_phase(const GatherArgs& g, int64_t
     }
   } else {
     s64 = __ldg(g.starts + b);
-    if (s64 >= g.len) s64 %= g.len;
+    s64 = window_start(s64, g.len);
     if (HASH && g.flags != nullptr && __ldg(g.flags + b) != 0) {
       const float* rec = A.rec + s64 * A.rec_stride;
       const int es = __float_as_int(__ldg(rec + A.col_ep_start)), ee = __float_as_int(__ldg(rec + A.col_ep_end));
@@ -1704,10 +1702,11 @@ int g_tile_ctas_per_sm = 0;  // tuning hook: resident tile-kernel blocks per SM 
 int g_force_generic_gather = 0;       // tests flip this to cover the descriptor-walking kernel
 int g_force_full_vector_relabel = 0;  // ... and this to cover MODE 1 with the bitflip functor
 
-int launch_gather(const fdql_arena* a, int64_t n, int64_t b_begin, int64_t b_end, int32_t T, int64_t len, const int64_t* starts, const uint8_t* flags,
-                         const int64_t* goal_rows, int32_t reward_op, const float* reward_params_host, int32_t n_params,
-                         double gamma, uint32_t opts, int32_t batch_for_weight, float* const* out, float* aux_mask,
-                         float* aux_contig, float* aux_weight, cudaStream_t st, const DrawSpec* draw) {
+// the fp32 keys, scalar records and aux of a gather (launch_gather adds the narrow keys)
+static int launch_gather_f32(const fdql_arena* a, int64_t n, int64_t b_begin, int64_t b_end, int32_t T, int64_t len, const int64_t* starts,
+                             const uint8_t* flags, const int64_t* goal_rows, int32_t reward_op, const float* reward_params_host,
+                             int32_t n_params, double gamma, uint32_t opts, int32_t batch_for_weight, float* const* out, float* aux_mask,
+                             float* aux_contig, float* aux_weight, cudaStream_t st, const DrawSpec* draw) {
   {
     const int rc = flush_pending_invalidation(a, st);
     if (rc) return rc;
@@ -2067,6 +2066,18 @@ int launch_gather(const fdql_arena* a, int64_t n, int64_t b_begin, int64_t b_end
 #undef FDQL_LAUNCH_GATHER
   FDQL_CUDA(cudaGetLastError());
   return FDQL_OK;
+}
+
+// The single router of every gather entry point: the fp32 gather, then (when it launched) the narrow keys' gather on the same stream
+// over the same windows -- the starts it was given, or the ones it drew (draw->starts_out) -- with the same modulus.
+int launch_gather(const fdql_arena* a, int64_t n, int64_t b_begin, int64_t b_end, int32_t T, int64_t len, const int64_t* starts,
+                  const uint8_t* flags, const int64_t* goal_rows, int32_t reward_op, const float* reward_params_host, int32_t n_params,
+                  double gamma, uint32_t opts, int32_t batch_for_weight, float* const* out, float* aux_mask, float* aux_contig,
+                  float* aux_weight, cudaStream_t st, const DrawSpec* draw) {
+  const int rc = launch_gather_f32(a, n, b_begin, b_end, T, len, starts, flags, goal_rows, reward_op, reward_params_host, n_params, gamma,
+                                   opts, batch_for_weight, out, aux_mask, aux_contig, aux_weight, st, draw);
+  if (rc != FDQL_OK) return rc;  // (1: this shape is not served by the drawing kernels, nothing launched, no starts drawn)
+  return launch_narrow_gather(a, n, b_begin, b_end, T, len, draw != nullptr ? draw->starts_out : starts, out, st);
 }
 
 }  // namespace fdql

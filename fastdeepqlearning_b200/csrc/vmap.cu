@@ -177,6 +177,9 @@ __global__ void __launch_bounds__(256) onehot_kernel(int64_t n_rows, int32_t n_a
 }
 
 static int vmap_keys(const fdql_arena* a, int32_t key_goals, int32_t key_rewards, int32_t key_dones, int32_t key_returns, VmapKeys* out) {
+  for (const int32_t key : {key_goals, key_rewards, key_dones, key_returns})
+    FDQL_REQUIRE(key < 0 || key >= a->n_keys || a->key_narrow[key] < 0,
+                 "key %d is stored as uint8 / int8: the virtual goal / reward / done / return keys must be fp32", key);
   auto slab = [&](int32_t key, WideSlab* w) -> bool {
     if (key < 0 || key >= a->n_keys || a->key_wide[key] < 0) return false;
     *w = a->dev.wide[a->key_wide[key]];

@@ -14,6 +14,8 @@
  *     own stream; the caller orders writer->reader with stream/event dependencies.
  *   - all learner-visible data is fp32, the dtype franQ's TorchDataLoader casts every key to
  *     (franQ/Replay/wrappers/torch_dataloader.py:36); row indices are int64 like numpy.random.randint.
+ *     Keys are stored as fp32 too, except "narrow" keys (fdql_arena_create_typed): a uint8 / int8 key is stored at one byte per
+ *     element, as franQ's ring keeps a numpy array's dtype, and every gather widens it to exact fp32 values (no scaling).
  */
 #ifndef FDQL_H_
 #define FDQL_H_
@@ -82,11 +84,34 @@ int fdql_version(void);
  *      width-1 keys are packed into one 16B-aligned scalar record per row next to the episode extents. ---- */
 int fdql_arena_create(int64_t capacity, int32_t n_keys, const int32_t* widths_host, const int32_t* roles_host,
                       int32_t device, fdql_arena** out);
+
+/* Storage types of fdql_arena_create_typed. */
+enum { FDQL_DTYPE_F32 = 0, FDQL_DTYPE_U8 = 1, FDQL_DTYPE_I8 = 2 };
+/* fdql_arena_create with a storage type per key (dtypes_host NULL: all FDQL_DTYPE_F32, which is fdql_arena_create).  A key of role
+ * NONE and width >= 2 may be FDQL_DTYPE_U8 or FDQL_DTYPE_I8, a "narrow key": one slab [capacity, stride] of bytes, stride = width
+ * rounded up to 16 (every row 16B-aligned).  Narrow keys are read and written only as follows:
+ *   - fdql_arena_append: src[k] is [n_rows, width] elements of the key's type; fdql_arena_append_host likewise from host memory;
+ *     fdql_arena_append_packed_host: the key's region of the packed row holds the raw bytes and is ceil(width/16)*4 floats wide;
+ *   - every gather (fdql_sample_gather, fdql_sample_gather_draw, fdql_fused_pass, fdql_fused_pass_per, fdql_gather_rows,
+ *     fdql_hotpath_step_host) writes out[k] as fp32 [T, n, width] (or [n, width]) holding the stored integers exactly (zero
+ *     extension for uint8, sign extension for int8), from the same rows as the fp32 keys of the call; it is one more launch on the
+ *     same stream after the fp32 gather (capturable like it);
+ *   - fdql_her_flush_episodes(_given) and fdql_q3_duplicate copy the narrow rows with the others;
+ *   - fdql_arena_narrow_view gives the raw slab.
+ * FDQL_EINVAL: an unknown dtype; a narrow dtype on a width-1 key or a key with a role.  fdql_arena_key_view refuses a narrow key, and
+ * fdql_vmap_flush_episodes(_given) / fdql_vmap_select_column refuse a narrow virtual key.  fdql_arena_info's bytes include the
+ * narrow slabs. */
+int fdql_arena_create_typed(int64_t capacity, int32_t n_keys, const int32_t* widths_host, const int32_t* roles_host,
+                            const int32_t* dtypes_host, int32_t device, fdql_arena** out);
+/* raw view of a narrow key: element (row, c) is the byte at base[row * row_stride_bytes + c], *dtype its FDQL_DTYPE_*.  FDQL_EINVAL
+ * for an fp32 key (use fdql_arena_key_view). */
+int fdql_arena_narrow_view(const fdql_arena* a, int32_t key, void** base, int64_t* row_stride_bytes, int32_t* dtype);
 int fdql_arena_destroy(fdql_arena* a);
 /* cursor state with the reference's arithmetic: top=(top+1)%capacity, len=max(top,len)  (replay_memory.py:45-46, Q1) */
 int fdql_arena_info(const fdql_arena* a, int64_t* capacity, int64_t* top, int64_t* len, int64_t* bytes);
 int fdql_arena_set_cursor(fdql_arena* a, int64_t top, int64_t len);
-/* raw view of one key's storage for zero-copy host-language views: element (row, c) lives at base[row*row_stride + col + c] */
+/* raw view of one fp32 key's storage for zero-copy host-language views: element (row, c) lives at base[row*row_stride + col + c]
+ * (FDQL_EINVAL for a narrow key: see fdql_arena_narrow_view) */
 int fdql_arena_key_view(const fdql_arena* a, int32_t key, float** base, int64_t* row_stride, int32_t* col);
 /* internal columns: which=0 ep_start(int32 bits), 1 ep_end(int32 bits) inside the scalar record; 2 goal-agnostic reward (column 2 of
  * the 16-byte scan records); 3 the 16-byte link records (column 0).  Used for zero-copy views and for snapshot / restore. */
